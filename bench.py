@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- IQ Msamples/s of the GPS L1 C/A synthesis hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--chan 32|12] [--iq16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--chan 32|12] [--iq16] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input: the
@@ -21,6 +21,8 @@ rank r synthesizes blocks [r*2999, (r+1)*2999) (weak scaling, no data-path colle
            counted (SURVEY.md section 8d).
   cpu_baseline / --impl reference: the reference's own producer loop (oracle/_ref/ref_run*,
            the unmodified gps.c behind a null sink) on this box's host cores.
+  --dump-outputs DIR: after the timed steps, what the last one computed (see dump_outputs), so that two builds
+           can be compared output for output; the inputs are seeded and identical from run to run.
 """
 import argparse
 import importlib
@@ -40,6 +42,7 @@ sys.path.insert(0, ROOT)
 NCU_DRAM_MB = {("k_synth", True): 98.34 + 303.58, ("k_synth_lanes", True): 98.39 + 319.31, ("k_synth_lanes", False): 61.84 + 317.22}
 BLOCKS_300S = 2999            # -d 300 -> round(10*300) - 1 blocks (gps.c:2703)
 SAMPLES_PER_BLOCK = 300000
+DUMP_BLOCKS = 16              # sampled blocks of --dump-outputs: at most 18 x 600000 float32 = 43.2 MB
 
 
 def note(msg):
@@ -260,6 +263,24 @@ def workload_config(nchan, iq16, gpus, stream_blocks, per_rank_blocks):
 BLOCKS_3600S = 35999          # BASELINE configs[4]: -d 3600
 
 
+def dump_outputs(dirname, out_dev, block_elems, phases, prefix=""):
+    """Write what a caller of the timed path receives from one step, as .npy:
+      carrier_phase.npy  float64 [channels]: the exact carrier phases at the end of the slice (all of them)
+      iq_sample.npy      float32 [n, block_elems]: whole blocks of the int8/int16 IQ stream (interleaved I, Q),
+                         a fixed, seeded sample of them (the stream is 1.8 GB for the default workload)
+      iq_sample_block.npy float64 [n]: the indices of those blocks in the slice (first and last always included)"""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    nblk = out_dev.numel() // block_elems
+    pick = np.random.default_rng(0).choice(nblk, size=min(DUMP_BLOCKS, nblk), replace=False)
+    pick = np.unique(np.concatenate([[0, nblk - 1], pick]))
+    iq = out_dev.view(nblk, block_elems)[torch.from_numpy(pick).to(out_dev.device)].float().cpu().numpy()
+    np.save(os.path.join(dirname, prefix + "carrier_phase.npy"), np.asarray(phases, dtype=np.float64))
+    np.save(os.path.join(dirname, prefix + "iq_sample.npy"), iq)
+    np.save(os.path.join(dirname, prefix + "iq_sample_block.npy"), pick.astype(np.float64))
+
+
 class HandOver:
     """The carrier-chain hand-over of a time-sliced stream over NCCL (include/gpsb200.h, "time-slice hand-over"):
     every step two small messages (32 satellite ids + 32 phases each) travel rank to rank with send/recv -- first the
@@ -339,7 +360,11 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not bind the rank to its GPU's NUMA node (A/B)")
     ap.add_argument("--run-samples", type=int, default=0, help="device work unit (0 = library default)")
     ap.add_argument("--depth", type=int, default=2, help="contexts used alternately by consecutive steps (1: no overlap)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/*.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -508,6 +533,9 @@ def main():
     if os.environ.get("BENCH_TRACE") and step_trace:
         note("step phases [prepare, links, probe, recv, finish+send | host_chain] ms: %s" % step_trace[-3:])
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs:                                     # before the replays below rewrite the buffer
+        dump_outputs(args.dump_outputs, out_dev, gps.BLOCK_ELEMS, ph_last, "rank%d_" % rank if world > 1 else "")
+        note("outputs of the last timed step written to %s" % args.dump_outputs)
     total_ms = max_over_ranks(total_ms)
     ms_per_step = total_ms / args.steps
     samples_all = total_blocks * SAMPLES_PER_BLOCK
@@ -540,7 +568,7 @@ def main():
         try:
             out_host = torch.empty(nblk * gps.BLOCK_ELEMS, dtype=torch.int16 if args.iq16 else torch.int8, pin_memory=True)
             out_np = out_host.numpy()
-            e2e_steps = max(3, min(args.steps, 8))      # PCIe throughput varies by a few % run to run
+            e2e_steps = args.steps
 
             def e2e_step():
                 if world == 1:          # the blocking public call: segmented pipeline, chain resolution of later

@@ -11,11 +11,11 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "ref: needs /root/reference and oracle/_ref reference binaries")
+    config.addinivalue_line("markers", "ref: needs the reference binaries of oracle/_ref (built only from the reference sources)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.exists("/root/reference/gps.c")
+    have_ref = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_sinkfeed"))
     for it in items:
         if "ref" in it.keywords and not have_ref:
-            it.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
+            it.add_marker(pytest.mark.skip(reason="oracle/_ref/ref_sinkfeed not built (needs the reference sources)"))

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """TEST INFRASTRUCTURE: (re)generate tests/golden/*.npz from the reference itself.
 
-Runs only where /root/reference and oracle/_ref/ref_dump{12,32} exist (the build
-container). For each scenario it runs the UNMODIFIED reference producer
+Runs only where oracle/Makefile has built the reference binaries (oracle/_ref/ref_*;
+that needs the reference sources). For each scenario it runs the UNMODIFIED reference producer
 (gps.c, gps_thread_ep) behind the recording FIFO of oracle/ref_harness/ref_dump.c
 and stores
   * the per-block channel parameters the sample loop consumed (f_carr, f_code,
@@ -26,6 +26,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import refdump  # noqa: E402
 
 REF = os.path.join(ROOT, "oracle", "_ref")
+CIRCLE = os.path.join(HERE, "circle.csv")   # the reference's own motion file, stored verbatim
 LOC = "35.681298,139.766247,10.0"
 START = "2024/01/07,02:00:00"   # = toc of the synthetic ephemerides (avoids date2gps on a zero date)
 
@@ -36,7 +37,7 @@ SCENARIOS = {
     # name: (nsat, binary, seconds, extra args, keep verbatim blocks)
     "sky12_static_10s_i8": (12, "ref_dump12", 10, [], [0, 98]),
     "sky12_static_35s_i8": (12, "ref_dump12", 35, [], []),
-    "sky12_circle_10s_i16": (12, "ref_dump12", 10, ["--iq16", "-m", "/root/reference/circle.csv"], [0]),
+    "sky12_circle_10s_i16": (12, "ref_dump12", 10, ["--iq16", "-m", CIRCLE], [0]),
     "sky32_static_10s_i8": (32, "ref_dump32", 10, [], [0]),
     # BASELINE configs[3]: motion file + --iq16 + 60 s; digests only (parameters come from the scenario engine)
     "sky12_track_60s_i16": (12, "ref_dump12", 60, ["--iq16", "-m", "@MOTION"], []),
@@ -51,7 +52,7 @@ SCENARIOS = {
 SCENARIOS["sky12_ephroll_400s_i8"] = (12, "ref_dump12", 400, [], [])
 # BASELINE configs[3] LITERALLY: the reference's own circle.csv, --iq16, 60 s (599 blocks). The motion rows the run
 # consumed travel inside the fixture (the GPU box has no /root/reference): tests re-write them with %.17g.
-SCENARIOS["sky12_circle_60s_i16"] = (12, "ref_dump12", 60, ["--iq16", "-m", "/root/reference/circle.csv"], [])
+SCENARIOS["sky12_circle_60s_i16"] = (12, "ref_dump12", 60, ["--iq16", "-m", CIRCLE], [])
 # ADALM-Pluto flavour of the sample loop: gain x 2 (gps.c:2759-2763), int16 (sdr_pluto.c:107-110)
 SCENARIOS["sky12_pluto_3s_i16"] = (12, "ref_dump12", 3, ["--iq16", "--pluto-gain"], [0])
 # -t distance,bearing,height: static start point relative to the location (gps.c:2348-2357)
@@ -116,8 +117,8 @@ def run(name):
         out["nav_frames"] = np.stack(frames)
         out["nav_frame_of_block"] = idx
         out.update(extra_out)
-        if "/root/reference/circle.csv" in extra:
-            rows = np.loadtxt("/root/reference/circle.csv", delimiter=",")
+        if CIRCLE in extra:
+            rows = np.loadtxt(CIRCLE, delimiter=",")
             out["motion_rows"] = rows[:int(secs * 10)]
         np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
         print(name, "blocks", nblk, "chan", p["max_chan"], "frames", len(frames),
@@ -148,6 +149,25 @@ def run_crc_only(name, nsat, binary, secs, crc_file=None):
 CRC_ONLY = {"sky32_static_3600s_i8": (32, "ref_run32_fast", 3600)}
 
 
+def run_stock(name, nsat, binary, secs):
+    """The reference program exactly as shipped (own fifo.c / sdr_iqfile.c): CRC-32 of every block of the
+    iqdata.bin it writes."""
+    with tempfile.TemporaryDirectory() as td:
+        nav = os.path.join(td, "sky.nav")
+        subprocess.check_call([sys.executable, os.path.join(ROOT, "oracle", "gen_rinex.py"),
+                               "--nsat", str(nsat), "--out", nav])
+        subprocess.check_call([os.path.join(REF, binary), "-e", nav, "-l", LOC, "-d", str(secs)], cwd=td,
+                              stderr=subprocess.DEVNULL, stdout=subprocess.DEVNULL)
+        crcs = refdump.block_crcs(np.fromfile(os.path.join(td, "iqdata.bin"), dtype=np.int8))[:, 0]
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), crcs=crcs, max_chan=np.int32(nsat), sample_size=np.int32(1),
+                        seconds=np.int32(secs))
+    print(name, "blocks", crcs.size)
+
+
+# configs[1] through the stock program: its FIFO loses buffers 1..6 (fifo.c:163-168)
+STOCK = {"sky12_static_10s_stock_iqfile": (12, "ref_stock12", 10)}
+
+
 if __name__ == "__main__":
     args = sys.argv[1:]
     crc_file = None
@@ -155,8 +175,10 @@ if __name__ == "__main__":
         i = args.index("--crc-file")
         crc_file = args[i + 1]
         del args[i:i + 2]
-    for n in (args or list(SCENARIOS) + list(CRC_ONLY)):
+    for n in (args or list(SCENARIOS) + list(CRC_ONLY) + list(STOCK)):
         if n in CRC_ONLY:
             run_crc_only(n, *CRC_ONLY[n], crc_file=crc_file)
+        elif n in STOCK:
+            run_stock(n, *STOCK[n])
         else:
             run(n)

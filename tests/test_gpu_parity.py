@@ -603,7 +603,7 @@ def test_reference_program_with_the_drop_in_patch_writes_the_reference_stream(tm
     import zlib
     exe = os.path.join(scenario.ROOT, "oracle", "_ref", "ref_gpsb200_12")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/ref_gpsb200_12 is built where /root/reference exists and travels with the snapshot")
+        pytest.skip("oracle/_ref/ref_gpsb200_12 not built (needs the reference sources)")
     nav = _nav_file(tmp_path, 12)
     g = scenario.load_golden("sky12_static_10s_i8")
     r = subprocess.run([exe, "-e", nav, "-l", "35.681298,139.766247,10.0", "-d", "10"], cwd=tmp_path,

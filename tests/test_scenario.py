@@ -31,13 +31,8 @@ def make_nav(tmp_path, nsat, v3=False, sets=1):
     return str(nav)
 
 
-def motion_file(tmp_path):
-    # the motion scenario was dumped with the reference's circle.csv; regenerate the same rows from
-    # the dump-independent source when it is available, else skip
-    src = "/root/reference/circle.csv"
-    if not os.path.exists(src):
-        pytest.skip("circle.csv travels only with /root/reference")
-    return src
+# the motion scenarios were dumped with the reference's circle.csv, stored verbatim in tests/golden
+CIRCLE = os.path.join(scenario.GOLD, "circle.csv")
 
 
 @pytest.mark.parametrize("name", list(CASES))
@@ -45,7 +40,7 @@ def test_scenario_engine_matches_reference_dump_bit_for_bit(name, tmp_path):
     c = CASES[name]
     g = scenario.load_golden(name)
     want, frames = scenario.golden_chans(g)
-    mot = motion_file(tmp_path) if c.get("motion") else None
+    mot = CIRCLE if c.get("motion") else None
     got, nav = gps.scenario(make_nav(tmp_path, c["nsat"], c.get("v3", False)), *LOC, seconds=c["secs"],
                             max_chan=c["chan"], motion_file=mot, start=START, rinex3=c.get("v3", False),
                             pluto_gain=c.get("pluto", False), target=c.get("target"))
@@ -155,10 +150,9 @@ def test_config3_circle_csv_60s_engine_matches_dump(tmp_path):
     assert got.shape == (599, 12)
     for f in ("prn", "iword", "ibit", "icode", "f_carr", "f_code", "code_phase", "gain"):
         assert np.array_equal(got[f][:2], g["chans"][f]), f
-    src = "/root/reference/circle.csv"
-    if os.path.exists(src):            # the re-written rows parse to the same doubles as the original file
-        ref, _ = gps.scenario(make_nav(tmp_path, 12), *LOC, seconds=60, max_chan=12, motion_file=src, start=START)
-        assert got.tobytes() == ref.tobytes()
+    # the re-written rows parse to the same doubles as the original file
+    ref, _ = gps.scenario(make_nav(tmp_path, 12), *LOC, seconds=60, max_chan=12, motion_file=CIRCLE, start=START)
+    assert got.tobytes() == ref.tobytes()
 
 
 def test_gzip_compressed_rinex_reads_like_the_plain_file(tmp_path):
