@@ -44,6 +44,19 @@ enum {
     GPSB200_ERR_INTERNAL = -5    /* device self-check failed (would mean a bug; never returns wrong samples silently) */
 };
 
+/* ---- carrier NCO of the reference build being replaced (gps.h:17) -------------------------------------------
+ * GPSB200_CARRIER_FP64 (default): `#define FLOAT_CARR_PHASE` present, as shipped: double carr_phase in [0,1),
+ *     carr_phase += f_carr * delt with a wrap per sample, table index floor(carr_phase * 512) (gps.c:2775, 2821-2826).
+ * GPSB200_CARRIER_U32: the define absent: unsigned int carr_phase, carr_phasestep = (int) round(512.0 * 65536.0 *
+ *     f_carr * delt) per block (gps.c:2745-2747), table index (carr_phase >> 16) & 511, carr_phase += carr_phasestep
+ *     modulo 2^32 per sample (gps.c:2777, 2828), allocation phase (unsigned int) (512.0 * 65536.0 * frac(phase_ini))
+ *     (gps.c:2212-2213). In a U32 context every carrier phase the API takes or returns (gpsb200_chan_t.carr_phase,
+ *     carr_phase_out, the slice calls' phase_in / phase_out / phase_guess_in, gpsb200_carrier_chain_device) is that
+ *     accumulator as an integer-valued double in [0, 2^32); any other value is GPSB200_ERR_ARG. The phase at any sample
+ *     is then a closed form, so these contexts launch no carrier-chain kernels at all. */
+#define GPSB200_CARRIER_FP64      0
+#define GPSB200_CARRIER_U32       1
+
 /* One channel for one 0.1 s block: the fields of the reference's channel_t
  * (gps.h:213-236) and gain[] (gps.c:2300) that the sample loop reads, as left by
  * computeCodePhase (gps.c:2033-2064) and the gain update (gps.c:2749-2763).
@@ -58,7 +71,7 @@ typedef struct gpsb200_chan {
     int32_t reserved;
     double f_carr;        /* Hz, Doppler (gps.c:2043); |f_carr| < 2.9 MHz */
     double f_code;        /* Hz (gps.c:2044); 0 < f_code <= 1.07 MHz */
-    double carr_phase;    /* cycles in [0,1): used for the first block of a call and whenever prn differs
+    double carr_phase;    /* cycles in [0,1) (GPSB200_CARRIER_U32: the u32 accumulator, see above): used for the first block of a call and whenever prn differs
                              from the previous block's prn in the same slot (allocateChannel, gps.c:2203-2210);
                              otherwise the phase is carried from the previous block (gps.c:2821-2826) */
     double code_phase;    /* chips in [0,1023) (gps.c:2049) */
@@ -72,6 +85,8 @@ typedef struct gpsb200_config {
     int32_t max_nav_frames;    /* NAV frames held at once (>= 1) */
     int32_t host_threads;      /* threads for the exact carrier-phase chain; 0 = auto */
     int32_t run_samples;       /* device work unit, divides 300000 and is a multiple of 32; 0 = default (2400) */
+    int32_t carrier_nco;       /* GPSB200_CARRIER_FP64 (0) or GPSB200_CARRIER_U32. Added last in version 0.3: callers
+                                  must be rebuilt against this header (the struct grew by 4 bytes) */
 } gpsb200_config_t;
 
 typedef struct gpsb200_ctx gpsb200_ctx_t;
@@ -192,14 +207,23 @@ int gpsb200_slice_link_host(const gpsb200_chan_t *chans, int nblk, int nchan, gp
 /* Host only: (prn_in, phase_in) -> guessed (prn_out, phase_out) after the slice `link` describes. */
 int gpsb200_link_apply(const gpsb200_slice_link_t *link, int nchan, const int32_t *prn_in, const double *phase_in,
                        int32_t *prn_out, double *phase_out);
+/* The same two for either carrier NCO (carrier_nco = GPSB200_CARRIER_FP64 / _U32; the two functions above are the FP64
+ * forms). U32: link.value is the EXACT advance over the slice modulo 2^32 (or, with reset_inside, the exact absolute
+ * phase after it), so gpsb200_link_apply_nco yields exact, not guessed, outgoing states; phases are u32 accumulators. */
+int gpsb200_slice_link_host_nco(const gpsb200_chan_t *chans, int nblk, int nchan, int carrier_nco,
+                                gpsb200_slice_link_t *link);
+int gpsb200_link_apply_nco(const gpsb200_slice_link_t *link, int nchan, int carrier_nco, const int32_t *prn_in,
+                           const double *phase_in, int32_t *prn_out, double *phase_out);
 
 /* Test hook of the device self-check: corrupt the resolved carrier chain of the next calls by one unit of the
- * rounding grid (on != 0); every synth call must then fail with GPSB200_ERR_INTERNAL instead of returning samples. */
+ * rounding grid (on != 0); every synth call must then fail with GPSB200_ERR_INTERNAL instead of returning samples.
+ * A GPSB200_CARRIER_U32 context has no carrier chain to corrupt: GPSB200_ERR_ARG. */
 int gpsb200_debug_corrupt_chain(gpsb200_ctx_t *ctx, int on);
 
 /* Name of the synthesis kernel a call with nchan channels launches on this context as it stands: "k_synth_lanes"
  * (lane = sample: run length a multiple of 96 up to 2400, every code rate seen so far within 1.0157 .. 1.0302 MHz, 16-byte aligned
- * destination, GPSB200_LANES != 0) or "k_synth" (lane = channel, no such conditions). Both are bit-exact; for reporting. */
+ * destination, GPSB200_LANES != 0) or "k_synth" (lane = channel, no such conditions); "k_synth_lanes_u32" / "k_synth_u32" in a
+ * GPSB200_CARRIER_U32 context (same selection rule). Both are bit-exact; for reporting. */
 const char *gpsb200_synth_kernel_name(const gpsb200_ctx_t *ctx, int nchan);
 
 /* Re-run the device part of the previous gpsb200_synth_blocks_device call (parameters,
@@ -209,13 +233,14 @@ int gpsb200_replay_device(gpsb200_ctx_t *ctx, void *dst_device, void *stream, in
 
 /* Exact carrier phase after n samples of Doppler f_carr (the chain of gps.c:2821-2826
  * without stepping every sample); host-only helper, also used by time-slice sharding
- * to seed a rank's first block. */
+ * to seed a rank's first block. FP64 carrier NCO only (the U32 one is u + n * step modulo 2^32). */
 double gpsb200_carrier_advance(double carr_phase, double f_carr, int64_t nsamples);
 
 /* Exact carrier phases after nblk blocks for every channel slot (same chaining rule as
  * gpsb200_synth_blocks; phase_in == NULL: block 0 takes chans[0][c].carr_phase, else
  * phase_in[c] continues a previous call). Host only, `threads` worker threads. A rank of a
- * time-slice sharded run calls this on the blocks BEFORE its slice to seed its first block. */
+ * time-slice sharded run calls this on the blocks BEFORE its slice to seed its first block.
+ * FP64 carrier NCO only (for U32 use gpsb200_slice_link_host_nco + gpsb200_link_apply_nco: exact). */
 int gpsb200_carrier_chain(const gpsb200_chan_t *chans, int nblk, int nchan, const double *phase_in,
                           double *phase_out, int threads);
 
@@ -243,7 +268,8 @@ int gpsb200_span_chain_host(const double *f_carr, int nblk, double start_true, d
 /* Host model of the lane = sample synthesis kernel (csrc/synth_lanes.h) for ONE block: the same window / band / repair
  * logic, executed on the CPU, int16 I/Q out. force bits: 1 = repair every sample's index, 2 = exact chip signs for every
  * window, 4 = every repair walks exactly from the run anchor, 8 = carry points of every window by the FP64 second
- * opinion instead of the 32-bit estimate. counters[4] = fast samples, repaired samples, exactly
+ * opinion instead of the 32-bit estimate, 16 = GPSB200_CARRIER_U32 (carr_phase / carr_out are u32 accumulators; the
+ * carrier index is exact, bits 1 and 4 do not apply). counters[4] = fast samples, repaired samples, exactly
  * rebuilt sign windows, exact walks. For tests (the algorithm against the oracle without a GPU); not a product path. */
 int gpsb200_lanes_model_block(const gpsb200_chan_t *chans, int nchan, const uint32_t *nav, int run_samples, int force,
                               int16_t *iq, double *carr_out, int64_t *counters);
@@ -272,7 +298,9 @@ typedef struct gpsb200_scenario_config {
     double start_sec;
     /* -t distance,bearing,height (gps-sim.c:145-148, gps.c:2348-2357): static runs start at a point given by distance
      * [m] and bearing [deg] from the location, height offset [m]; ignored with a motion file, as in the reference */
-    int32_t target_valid, reserved;
+    int32_t target_valid;
+    int32_t carrier_u32;           /* 1: allocation phases of the reference's integer carrier build (gps.c:2212-2213),
+                                      carr_phase = (unsigned int) (512.0 * 65536.0 * frac(phase_ini)); 0: FP64 build */
     double target_distance_m, target_bearing_deg, target_height_m;
 } gpsb200_scenario_config_t;
 typedef struct gpsb200_scenario gpsb200_scenario_t;

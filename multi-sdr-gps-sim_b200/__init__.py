@@ -10,6 +10,7 @@ Import it with importlib (the directory name is not a Python identifier):
 from .api import (  # noqa: F401
     BLOCK_ELEMS, BLOCK_SAMPLES, SC08, SC16, Chan, Config, Context, GpsB200Error, Stats,
     bind_numa, carrier_advance, span_chain_host, lanes_model_block, link_apply, slice_link_host, SliceLink, carrier_chain, codegen, scenario, lib, lib_path, CHAN_DTYPE,
+    CARRIER_FP64, CARRIER_U32, carrier_advance_u32,
 )
 from .synthetic import synthetic_chans  # noqa: F401,E402
 from . import sharding  # noqa: F401,E402

@@ -1,6 +1,7 @@
 """ctypes mirror of include/gpsb200.h. No compute happens here and there is no CPU
 fallback: if libgpsb200.so is missing or no CUDA device is present the calls fail."""
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -8,6 +9,19 @@ import numpy as np
 BLOCK_SAMPLES = 300000
 BLOCK_ELEMS = 600000
 SC08, SC16 = 1, 2
+CARRIER_FP64, CARRIER_U32 = 0, 1     # gpsb200_config_t.carrier_nco
+_CARRIER = {"fp64": CARRIER_FP64, "u32": CARRIER_U32}
+
+
+def carrier_nco(carrier):
+    """'fp64' | 'u32' (or the GPSB200_CARRIER_* value) -> GPSB200_CARRIER_* value."""
+    if isinstance(carrier, str):
+        if carrier not in _CARRIER:
+            raise ValueError("carrier must be 'fp64' or 'u32', not %r" % carrier)
+        return _CARRIER[carrier]
+    if carrier not in (CARRIER_FP64, CARRIER_U32):
+        raise ValueError("bad carrier NCO %r" % (carrier,))
+    return int(carrier)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -39,7 +53,8 @@ assert CHAN_DTYPE.itemsize == C.sizeof(Chan) == 64
 
 class Config(C.Structure):
     _fields_ = [("device", C.c_int32), ("max_chan", C.c_int32), ("max_blocks", C.c_int32),
-                ("max_nav_frames", C.c_int32), ("host_threads", C.c_int32), ("run_samples", C.c_int32)]
+                ("max_nav_frames", C.c_int32), ("host_threads", C.c_int32), ("run_samples", C.c_int32),
+                ("carrier_nco", C.c_int32)]
 
 
 class ScenarioConfig(C.Structure):
@@ -49,7 +64,7 @@ class ScenarioConfig(C.Structure):
                 ("pluto_gain", C.c_int32),
                 ("start_year", C.c_int32), ("start_month", C.c_int32), ("start_day", C.c_int32),
                 ("start_hour", C.c_int32), ("start_min", C.c_int32), ("rinex3", C.c_int32),
-                ("start_sec", C.c_double), ("target_valid", C.c_int32), ("reserved", C.c_int32),
+                ("start_sec", C.c_double), ("target_valid", C.c_int32), ("carrier_u32", C.c_int32),
                 ("target_distance_m", C.c_double), ("target_bearing_deg", C.c_double), ("target_height_m", C.c_double)]
 
 
@@ -75,7 +90,8 @@ EXPORTS = ["gpsb200_create", "gpsb200_destroy", "gpsb200_last_error", "gpsb200_v
            "gpsb200_synth_blocks", "gpsb200_synth_blocks_scatter", "gpsb200_synth_blocks_device", "gpsb200_replay_device",
            "gpsb200_carrier_advance", "gpsb200_carrier_chain", "gpsb200_carrier_chain_device", "gpsb200_carrier_probe_fixup",
            "gpsb200_codegen", "gpsb200_bind_numa", "gpsb200_span_chain_host", "gpsb200_lanes_model_block", "gpsb200_slice_prepare", "gpsb200_slice_probe",
-           "gpsb200_slice_finish", "gpsb200_slice_finish_cb", "gpsb200_slice_wait", "gpsb200_link_apply", "gpsb200_slice_link_host", "gpsb200_debug_corrupt_chain", "gpsb200_synth_kernel_name",
+           "gpsb200_slice_finish", "gpsb200_slice_finish_cb", "gpsb200_slice_wait", "gpsb200_link_apply", "gpsb200_slice_link_host",
+           "gpsb200_link_apply_nco", "gpsb200_slice_link_host_nco", "gpsb200_debug_corrupt_chain", "gpsb200_synth_kernel_name",
            "gpsb200_scenario_create", "gpsb200_scenario_destroy", "gpsb200_scenario_error",
            "gpsb200_scenario_blocks", "gpsb200_scenario_channels", "gpsb200_scenario_nav_frames",
            "gpsb200_scenario_chans", "gpsb200_scenario_nav",
@@ -127,6 +143,9 @@ def lib():
         L.gpsb200_slice_probe.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.gpsb200_slice_finish.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(Stats)]
         L.gpsb200_link_apply.argtypes = [C.POINTER(SliceLink), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.gpsb200_slice_link_host_nco.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(SliceLink)]
+        L.gpsb200_link_apply_nco.argtypes = [C.POINTER(SliceLink), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p]
         L.gpsb200_debug_corrupt_chain.argtypes = [C.c_void_p, C.c_int]
         L.gpsb200_synth_kernel_name.argtypes = [C.c_void_p, C.c_int]
         L.gpsb200_synth_kernel_name.restype = C.c_char_p
@@ -167,9 +186,11 @@ def carrier_chain(chans, phase_in=None, threads=16):
     return out
 
 
-def lanes_model_block(chans_row, nav_frame, run_samples=2400, force=0):
+def lanes_model_block(chans_row, nav_frame, run_samples=2400, force=0, carrier="fp64"):
     """Host model of the lane = sample kernel for one block. chans_row: CHAN_DTYPE[nchan]; nav_frame: uint32[nchan, 60].
-    -> (iq int16[600000], carr_out float64[nchan], counters int64[4])"""
+    carrier='u32' sets force bit 16 (integer carrier NCO). -> (iq int16[600000], carr_out float64[nchan], counters int64[4])"""
+    if carrier_nco(carrier) == CARRIER_U32:
+        force |= 16
     a = np.ascontiguousarray(chans_row, dtype=CHAN_DTYPE)
     nv = np.ascontiguousarray(nav_frame, dtype=np.uint32)
     iq = np.zeros(BLOCK_ELEMS, np.int16)
@@ -195,32 +216,47 @@ def span_chain_host(f_carr, start_true, start_guess):
     return out if rc == 1 else None
 
 
-def slice_link_host(chans):
-    """gpsb200_slice_link_host: the closed-form link of a slice (host only). -> SliceLink"""
+def slice_link_host(chans, carrier="fp64"):
+    """gpsb200_slice_link_host_nco: the closed-form link of a slice (host only; exact for carrier='u32'). -> SliceLink"""
     a = np.ascontiguousarray(chans, dtype=CHAN_DTYPE)
     link = SliceLink()
-    rc = lib().gpsb200_slice_link_host(a.ctypes.data, a.shape[0], a.shape[1], C.byref(link))
+    rc = lib().gpsb200_slice_link_host_nco(a.ctypes.data, a.shape[0], a.shape[1], carrier_nco(carrier), C.byref(link))
     if rc:
-        raise GpsB200Error(rc, "gpsb200_slice_link_host")
+        raise GpsB200Error(rc, "gpsb200_slice_link_host_nco")
     return link
 
 
-def link_apply(link, nchan, prn_in=None, phase_in=None):
-    """gpsb200_link_apply -> (prn_out int32[nchan], phase_out float64[nchan])."""
+def link_apply(link, nchan, prn_in=None, phase_in=None, carrier="fp64"):
+    """gpsb200_link_apply_nco -> (prn_out int32[nchan], phase_out float64[nchan])."""
     pi = None if prn_in is None else np.ascontiguousarray(prn_in, dtype=np.int32)
     xi = None if phase_in is None else np.ascontiguousarray(phase_in, dtype=np.float64)
     po, xo = np.zeros(nchan, np.int32), np.zeros(nchan, np.float64)
-    rc = lib().gpsb200_link_apply(C.byref(link), nchan, None if pi is None else pi.ctypes.data,
-                                  None if xi is None else xi.ctypes.data, po.ctypes.data, xo.ctypes.data)
+    rc = lib().gpsb200_link_apply_nco(C.byref(link), nchan, carrier_nco(carrier), None if pi is None else pi.ctypes.data,
+                                      None if xi is None else xi.ctypes.data, po.ctypes.data, xo.ctypes.data)
     if rc:
-        raise GpsB200Error(rc, "gpsb200_link_apply")
+        raise GpsB200Error(rc, "gpsb200_link_apply_nco")
     return po, xo
 
 
+def carrier_advance_u32(u, f_carr, n):
+    """The reference's integer carrier NCO (gps.c:2746, 2828) on the host, for tests: u + n * carr_phasestep modulo
+    2^32, carr_phasestep = (int) round(512.0 * 65536.0 * f_carr * delt) evaluated in the reference's order."""
+    return float((int(u) + int(n) * _u32_step(f_carr)) % (1 << 32))
+
+
+def _u32_step(f_carr):
+    x = (33554432.0 * float(f_carr)) * (1.0 / 3000000.0)
+    ax = abs(x)
+    r = math.floor(ax)
+    r += 1 if ax - r >= 0.5 else 0                       # C round(): ties away from zero (ax - r is exact)
+    return int(r) if x >= 0 else -int(r)
+
+
 def scenario(nav_file, lat, lon, height, seconds, max_chan=12, motion_file=None, start=None,
-             ionosphere=True, pluto_gain=False, rinex3=False, target=None):
+             ionosphere=True, pluto_gain=False, rinex3=False, target=None, carrier="fp64"):
     """Run the host scenario engine. -> (chans[nblk, max_chan] CHAN_DTYPE, nav[nframes, max_chan, 60] uint32).
-    start: (y, m, d, hh, mm, sec) or None for the first ephemeris epoch."""
+    start: (y, m, d, hh, mm, sec) or None for the first ephemeris epoch. carrier='u32': allocation phases of the
+    reference's integer carrier build (u32 accumulators)."""
     cfg = ScenarioConfig()
     cfg.nav_file = os.fsencode(nav_file)
     cfg.motion_file = os.fsencode(motion_file) if motion_file else None
@@ -230,6 +266,7 @@ def scenario(nav_file, lat, lon, height, seconds, max_chan=12, motion_file=None,
     cfg.ionosphere_enable = 1 if ionosphere else 0
     cfg.pluto_gain = 1 if pluto_gain else 0
     cfg.rinex3 = 1 if rinex3 else 0
+    cfg.carrier_u32 = 1 if carrier_nco(carrier) == CARRIER_U32 else 0
     if target is not None:          # -t distance,bearing,height
         cfg.target_valid = 1
         cfg.target_distance_m, cfg.target_bearing_deg, cfg.target_height_m = [float(v) for v in target]
@@ -255,9 +292,12 @@ def scenario(nav_file, lat, lon, height, seconds, max_chan=12, motion_file=None,
 class Context:
     """gpsb200_ctx_t. `chans` arguments are numpy arrays of CHAN_DTYPE shaped [nblk, nchan]."""
 
-    def __init__(self, max_chan, max_blocks, device=0, max_nav_frames=1, host_threads=0, run_samples=0):
+    def __init__(self, max_chan, max_blocks, device=0, max_nav_frames=1, host_threads=0, run_samples=0, carrier="fp64"):
+        """carrier: 'fp64' (the reference as shipped) or 'u32' (its integer carrier NCO build); in a 'u32' context
+        every carrier phase in or out is the u32 accumulator as an integer-valued float."""
         self._h = C.c_void_p()
-        self.cfg = Config(device, max_chan, max_blocks, max_nav_frames, host_threads, run_samples)
+        self.carrier = "u32" if carrier_nco(carrier) == CARRIER_U32 else "fp64"
+        self.cfg = Config(device, max_chan, max_blocks, max_nav_frames, host_threads, run_samples, carrier_nco(carrier))
         rc = lib().gpsb200_create(C.byref(self.cfg), C.byref(self._h))
         if rc:
             msg = lib().gpsb200_last_error(self._h).decode() if self._h else "gpsb200_create: bad configuration"

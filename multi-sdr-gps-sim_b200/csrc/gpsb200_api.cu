@@ -144,6 +144,8 @@ struct gpsb200_ctx {
     double *d_blk_shift = nullptr, *h_blk_shift = nullptr;     // host-resolved spans: per-block shift / variant pick
     int32_t *d_blk_pick = nullptr, *h_blk_pick = nullptr;
     int run_ld = 0;                                    // leading dimension (blocks, padded) of d_run_x
+    bool u32 = false;                                  // cfg.carrier_nco == GPSB200_CARRIER_U32: exact closed-form carrier,
+                                                       // none of the carrier-chain stages (probes, chaining, scan) run
     bool lanes_on = true;                              // GPSB200_LANES=0: always k_synth (lane = channel)
     bool lanes_veto = false;                           // a channel record outside k_synth_lanes' range was seen
     int check_stride = 8, check_phase = 0;             // sampled exact re-walk of the chain (GPSB200_CHECK_STRIDE)
@@ -225,26 +227,34 @@ inline uint64_t step_to_fix(double c) {     // c in (-1, 1): c * 2^64 modulo 2^6
     return c < 0.0 ? (uint64_t) 0 - m : m;
 }
 
+inline bool valid_u32_phase(double p) { return p >= 0.0 && p < 4294967296.0 && p == std::floor(p); }
+
 // With link != NULL (time-slice hand-over, gpsb200_slice_prepare) the incoming chain state is not known yet:
 // guesses are accumulated RELATIVE to it (h_guess holds the advance since the slice start, h_guess_abs marks
 // blocks after a (re)allocation inside the slice, whose guesses are absolute) and finalize_guesses() adds the
 // offset later; *link describes how the slice maps an incoming state to the guessed outgoing one.
 // end_guess (optional): the GUESSED chain state after block b1-1, to seed the guesses of the next segment when that
 // is prepared before this one has been resolved.
+// U32 contexts: the same pass computes every block's carr_phasestep and its EXACT start phase (a modular prefix sum that
+// restarts from carr_phase whenever the slot's satellite changes); with link != NULL the start phases of blocks before
+// the slot's first (re)allocation are relative to the incoming phase (h_guess_abs == 0) until u32_rebase().
 int prepare_blocks(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1, int nchan,
                    const std::vector<ChainState> &chain, gpsb200_slice_link_t *link = nullptr,
                    std::vector<ChainState> *end_guess = nullptr) {
     const double delt = 1.0 / (double) GPSB200_SAMPLERATE;     // gps.c:2298
+    const bool u32 = ctx->u32;
     std::vector<int> status(nchan, GPSB200_OK);
     std::vector<uint8_t> lanes_bad(nchan, 0);
     ctx->pool->run(nchan, [&](int c_lo, int c_hi) {
         for (int c = c_lo; c < c_hi; c++) {
             // phase accumulator in cycles * 2^64, modulo 2^64 (= modulo one cycle): exact integer arithmetic
             uint64_t acc = phase_to_fix(chain[c].phase);    // exact phase after block b0-1 (if any)
+            uint32_t uacc = u32 ? (uint32_t) chain[c].phase : 0u;   // U32: exact phase after block b0-1
             int prev_prn = chain[c].prn;                    // 0 at the start of a call: block 0 is "fresh"
             bool absolute = link == nullptr;                // relative mode: true once a slot was (re)allocated
             if (link) {
                 acc = 0;
+                uacc = 0u;
                 prev_prn = chans[(size_t) b0 * nchan + c].prn;      // block b0 continues whatever comes in (decided later)
                 link->prn_first[c] = prev_prn;
                 link->first_phase[c] = prev_prn > 0 ? chans[(size_t) b0 * nchan + c].carr_phase : 0.0;
@@ -283,25 +293,32 @@ int prepare_blocks(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1
                     return;
                 }
                 // a slot whose satellite changed (or the first block of a call): the caller's carr_phase applies
-                if (!(in.carr_phase >= 0.0 && in.carr_phase < 1.0)) {      // read whenever a slot takes a new satellite
-                    status[c] = GPSB200_ERR_ARG;
+                if (!(u32 ? valid_u32_phase(in.carr_phase) : (in.carr_phase >= 0.0 && in.carr_phase < 1.0))) {
+                    status[c] = GPSB200_ERR_ARG;      // read whenever a slot takes a new satellite
                     return;
                 }
                 if (in.prn != prev_prn) {
                     acc = phase_to_fix(in.carr_phase);
+                    uacc = u32 ? (uint32_t) in.carr_phase : 0u;
                     absolute = true;
                 }
                 ctx->h_guess_abs[i] = absolute ? 1 : 0;
                 prev_prn = in.prn;
                 o.c_carr = in.f_carr * delt;                    // gps.c:2821
                 o.c_code = in.f_code * delt;                    // gps.c:2789
-                if (!lanes::code_step_ok(o.c_code) || !(std::fabs(o.c_carr) < 0.5)) lanes_bad[c] = 1;
+                if (!lanes::code_step_ok(o.c_code) || (!u32 && !(std::fabs(o.c_carr) < 0.5))) lanes_bad[c] = 1;
                 o.gain = in.gain;
                 o.carr_in = in.carr_phase;
                 o.code0 = in.code_phase;
                 o.prn = in.prn;
                 o.nav0 = (uint32_t) in.iword | ((uint32_t) in.ibit << 8) | ((uint32_t) in.icode << 16);
                 o.frame = in.nav_frame;
+                if (u32) {
+                    o.step_u32 = lanes::u32_carrier_step(in.f_carr);
+                    o.u0 = uacc;
+                    uacc += (uint32_t) GPSB200_BLOCK_SAMPLES * (uint32_t) o.step_u32;     // gps.c:2828, modulo 2^32
+                    continue;
+                }
                 ctx->h_guess[i] = fix_to_phase(acc);
                 // one block: 300000 steps of c, plus the expected rounding drift of those steps. (The drift of a block is
                 // up to +-8e-12 cycles and depends on the low bits of c, i.e. it is uncorrelated from block to block:
@@ -309,14 +326,15 @@ int prepare_blocks(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1
                 acc += (uint64_t) GPSB200_BLOCK_SAMPLES * step_to_fix(o.c_carr);
                 acc += (uint64_t) (int64_t) ((double) GPSB200_BLOCK_SAMPLES * carrier_drift_per_step(o.c_carr) * 0x1p64);
             }
+            const double end_phase = u32 ? (double) uacc : fix_to_phase(acc);
             if (end_guess) {
                 (*end_guess)[c].prn = prev_prn > 0 ? prev_prn : 0;
-                (*end_guess)[c].phase = prev_prn > 0 ? fix_to_phase(acc) : 0.0;
+                (*end_guess)[c].phase = prev_prn > 0 ? end_phase : 0.0;
             }
             if (link) {
                 link->prn_last[c] = prev_prn > 0 ? prev_prn : 0;
                 link->reset_inside[c] = absolute ? 1 : 0;
-                link->value[c] = fix_to_phase(acc);
+                link->value[c] = end_phase;
             }
         }
     });
@@ -334,6 +352,38 @@ int prepare_blocks(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1
         if (amp > 32767.0) return fail(ctx, GPSB200_ERR_RANGE, "sum of channel amplitudes exceeds int16 range");
     }
     return GPSB200_OK;
+}
+
+// U32: the exact chain state after block b1-1, straight from the prepared records (closed form).
+void u32_chain_end(const gpsb200_ctx *ctx, int b1, int nchan, std::vector<ChainState> &chain) {
+    for (int c = 0; c < nchan; c++) {
+        const BlockChanDev &p = ctx->h_bc[(size_t) (b1 - 1) * nchan + c];
+        chain[c].prn = p.prn > 0 ? p.prn : 0;
+        chain[c].phase = p.prn > 0 ? (double) (p.u0 + (uint32_t) GPSB200_BLOCK_SAMPLES * (uint32_t) p.step_u32) : 0.0;
+    }
+}
+
+// U32, relative mode of a slice: the exact incoming state is known now; move the start phases of the blocks before each
+// slot's first (re)allocation from "advance since the slice start" to absolute (same rule as finalize_guesses).
+void u32_rebase(gpsb200_ctx *ctx, int nblk, int nchan, const int32_t *prn_in, const double *phase_in) {
+    for (int c = 0; c < nchan; c++) {
+        const BlockChanDev &first = ctx->h_bc[c];
+        const bool cont = prn_in && phase_in && first.prn > 0 && prn_in[c] == first.prn;
+        const uint32_t off = (uint32_t) (cont ? phase_in[c] : first.carr_in);
+        for (int b = 0; b < nblk; b++) {
+            const size_t i = (size_t) b * nchan + c;
+            if (ctx->h_guess_abs[i] || ctx->h_bc[i].prn <= 0) continue;
+            ctx->h_bc[i].u0 += off;
+        }
+    }
+}
+
+// Incoming carrier phases a caller hands in (slots with prn_in > 0): [0,1) for FP64, u32 accumulators for U32.
+bool phases_ok(const gpsb200_ctx *ctx, int nchan, const int32_t *prn_in, const double *phase_in) {
+    if (!prn_in || !phase_in) return true;
+    for (int c = 0; c < nchan; c++)
+        if (prn_in[c] > 0 && !(ctx->u32 ? valid_u32_phase(phase_in[c]) : (phase_in[c] >= 0.0 && phase_in[c] < 1.0))) return false;
+    return true;
 }
 
 // Second pass of the relative mode: the (guessed) incoming state is known now.
@@ -509,6 +559,7 @@ void fill_args(gpsb200_ctx *ctx, SynthArgs &a, int blk0, int nblk, int nchan, in
     a.blk_shift = ctx->d_blk_shift + off;
     a.blk_pick = ctx->d_blk_pick + off;
     a.lanes = ctx->lanes_on && !ctx->lanes_veto ? 1 : 0;
+    a.u32 = ctx->u32 ? 1 : 0;
     // lanes per run follow the channel count; a CTA takes up to 24 warps' worth of runs
     const int grp = nchan > 16 ? 32 : (nchan > 8 ? 16 : 8);
     const int rpw = 32 / grp;
@@ -570,6 +621,7 @@ int segment_params(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1
 // Second part: everything speculative -- guesses up, block probes, span chaining. Needs no true start phase.
 int segment_probe(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
                   const SynthArgs &a) {
+    if (ctx->u32) return GPSB200_OK;                 // exact closed form: nothing to speculate about
     const size_t off = (size_t) b0 * nchan, cnt = (size_t) (b1 - b0) * nchan;
     CU(cudaMemcpyAsync(ctx->d_guess + off, ctx->h_guess + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
     if (first) CU(cudaEventRecord(ctx->ev[1], sp));
@@ -590,6 +642,14 @@ int segment_checkpoints(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_
 int segment_resolve(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, std::vector<ChainState> &chain,
                     gpsb200_stats_t &st, bool first, const SynthArgs &a, cudaEvent_t probes_done = nullptr,
                     int64_t *slow_out = nullptr) {
+    if (ctx->u32) {                 // the exact state is a closed form of the prepared records: no probes to wait for
+        u32_chain_end(ctx, b1, nchan, chain);
+        if (slow_out) {
+            *slow_out = 0;
+            return GPSB200_OK;
+        }
+        return segment_checkpoints(ctx, b0, b1, nchan, sp, st, first, a, 0);
+    }
     // probes and span summaries must be in (mapped) host memory: wait for the segment's own probe event when the
     // post-scan work runs on a stream of its own (slice path), else for the pre-phase stream
     if (probes_done) CU(cudaEventSynchronize(probes_done));
@@ -611,8 +671,10 @@ int segment_checkpoints(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_
     const size_t off = (size_t) b0 * nchan, cnt = (size_t) (b1 - b0) * nchan;
     const size_t soff = (size_t) (b0 / kSpanBlocks) * nchan, scnt = (size_t) a.nspan * nchan;
     if (first) CU(cudaEventRecord(ctx->ev[3], sp));
-    CU(cudaMemcpyAsync(ctx->d_span_res + soff, ctx->h_span_res + soff, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
-    st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
+    if (!ctx->u32) {                                 // U32: k_checkpoints reads no span resolutions
+        CU(cudaMemcpyAsync(ctx->d_span_res + soff, ctx->h_span_res + soff, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
+        st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
+    }
     if (slow > 0) {                                  // rare: per-block resolutions of the host-resolved spans
         CU(cudaMemcpyAsync(ctx->d_carr0 + off, ctx->h_carr0 + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
         CU(cudaMemcpyAsync(ctx->d_blk_shift + off, ctx->h_blk_shift + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
@@ -694,12 +756,13 @@ int small_call(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int ncha
                 }
                 if (stc.prn != p.prn) stc.phase = p.carr_in;
                 stc.prn = p.prn;
-                double x = stc.phase, y = p.code0;
+                double x = ctx->u32 ? (double) p.u0 : stc.phase, y = p.code0;
                 int iword = p.nav0 & 0xFF, ibit = (p.nav0 >> 8) & 0xFF, icode = (p.nav0 >> 16) & 0xFF;
                 for (int r = 0; r < nruns; r++) {
                     ck[(size_t) r * nchan] = RunCkpt{x, y, (uint32_t) iword | ((uint32_t) ibit << 8) | ((uint32_t) icode << 16), 0u};
                     int64_t periods = 0, dummy = 0;
-                    nco_advance<NCO_CARRIER>(x, p.c_carr, run, dummy);
+                    if (ctx->u32) x = (double) ((uint32_t) x + (uint32_t) run * (uint32_t) p.step_u32);     // gps.c:2828
+                    else nco_advance<NCO_CARRIER>(x, p.c_carr, run, dummy);
                     nco_advance<NCO_CODE>(y, p.c_code, run, periods);
                     nav_advance(iword, ibit, icode, periods);
                 }
@@ -829,7 +892,8 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
         }
         int64_t slow = 0;
         trace(ctx, "speculative work enqueued");
-        for (size_t i = 0; i < segs.size(); i++) {
+        if (ctx->u32) chain = guess;                    // U32: the prepared end state is exact
+        for (size_t i = 0; i < segs.size() && !ctx->u32; i++) {
             CU(cudaEventSynchronize(ctx->ev_seg[std::min((int) i, ctx->max_segs - 1)]));
             const double t0 = now_ms();
             int64_t reg = 0, sl = 0;
@@ -843,7 +907,7 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
         fill_args(ctx, all, 0, nblk, nchan, sample_size, dst_dev);
         const size_t cnt = (size_t) nblk * nchan, scnt = (size_t) all.nspan * nchan;
         CU(cudaEventRecord(ctx->ev[3], sp));
-        CU(cudaMemcpyAsync(ctx->d_span_res, ctx->h_span_res, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
+        if (!ctx->u32) CU(cudaMemcpyAsync(ctx->d_span_res, ctx->h_span_res, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
         if (slow > 0) {
             CU(cudaMemcpyAsync(ctx->d_carr0, ctx->h_carr0, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
             CU(cudaMemcpyAsync(ctx->d_blk_shift, ctx->h_blk_shift, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
@@ -860,7 +924,7 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
         CU(cudaStreamWaitEvent(s, ctx->ev_done[0], 0));
         CU(launch_synth(all, s));
         st.launches += 2;
-        st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
+        if (!ctx->u32) st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
         trace(ctx, "checkpoints + synthesis enqueued");
     }
     for (const auto &sg : segs) {
@@ -906,8 +970,10 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
     if (stats) {
         float ms = 0;
         // per-kernel times of the FIRST segment ...
-        cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]);
-        st.probe_kernel_ms = ms;
+        if (!ctx->u32) {    // (a U32 call records no probe events)
+            cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]);
+            st.probe_kernel_ms = ms;
+        }
         cudaEventElapsedTime(&ms, ctx->ev[3], ctx->ev[4]);
         st.checkpoint_kernel_ms = ms;
         if (dst_host) {      // ... and the whole span of the call's stream (a device-destination call is still running)
@@ -936,7 +1002,7 @@ int run_pipeline(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int nc
 
 extern "C" {
 
-const char *gpsb200_version(void) { return "gpsb200 0.2 (sm_100a)"; }
+const char *gpsb200_version(void) { return "gpsb200 0.3 (sm_100a)"; }
 
 int gpsb200_bind_numa(int device) {
     char bus[32] = {0};
@@ -1080,11 +1146,13 @@ int gpsb200_create(const gpsb200_config_t *cfg, gpsb200_ctx_t **out) {
     if (c.host_threads <= 0) c.host_threads = (int) std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
     if (c.max_nav_frames <= 0) c.max_nav_frames = 1;
     if (c.max_chan < 1 || c.max_chan > GPSB200_MAX_CHAN || c.max_blocks < 1 || c.run_samples < 32 ||
-        c.run_samples % 32 != 0 || GPSB200_BLOCK_SAMPLES % c.run_samples != 0) {
+        c.run_samples % 32 != 0 || GPSB200_BLOCK_SAMPLES % c.run_samples != 0 ||
+        (c.carrier_nco != GPSB200_CARRIER_FP64 && c.carrier_nco != GPSB200_CARRIER_U32)) {
         delete ctx;
         return GPSB200_ERR_ARG;
     }
     ctx->nruns = GPSB200_BLOCK_SAMPLES / c.run_samples;
+    ctx->u32 = c.carrier_nco == GPSB200_CARRIER_U32;
     if (const char *ev = getenv("GPSB200_GRADED_CHUNKS")) ctx->graded_chunks = atoi(ev) != 0;
     ctx->pool.reset(new WorkerPool(std::min(c.host_threads, c.max_chan)));
     *out = ctx;   // from here on errors are reported through the context
@@ -1298,11 +1366,17 @@ int gpsb200_slice_probe(gpsb200_ctx_t *ctx, const int32_t *prn_in, const double 
         return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_probe: call gpsb200_slice_prepare first");
     CU(cudaSetDevice(ctx->cfg.device));
     const int nblk = ctx->pending.nblk, nchan = ctx->pending.nchan;
+    if (!phases_ok(ctx, nchan, prn_in, phase_guess_in))
+        return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_probe: phase_guess_in is not a carrier phase of this context");
+    ctx->pending.eager = eager != 0;
+    if (ctx->u32) {                  // exact closed form: nothing speculative to enqueue
+        ctx->pending.probed = true;
+        return GPSB200_OK;
+    }
     const double t0 = now_ms();
     finalize_guesses(ctx, 0, nblk, nchan, prn_in, phase_guess_in);
     ctx->pending.st.host_chain_ms += now_ms() - t0;
     int rc = GPSB200_OK, iseg = 0;
-    ctx->pending.eager = eager != 0;
     const auto segs = segments_of(nblk);
     if (ctx->pending.eager) {
         // everything speculative at once: ONE probe and ONE chaining launch over the whole slice (no per-segment tails)
@@ -1340,6 +1414,49 @@ int slice_finish_inner(gpsb200_ctx *ctx, std::vector<ChainState> &chain, gpsb200
     std::vector<std::vector<ChainState>> after(segs.size());
     ctx->trace_t0 = now_ms();
     trace(ctx, "slice_finish");
+    if (ctx->u32) {
+        // The exact outgoing state is a closed form: hand it over at once, then enqueue per segment the corrected
+        // parameters' run checkpoints and the synthesis.
+        std::vector<ChainState> in = chain;
+        std::vector<int32_t> pi(nchan);
+        std::vector<double> xi(nchan);
+        export_chain(in, nchan, pi.data(), xi.data());
+        CU(cudaStreamSynchronize(ctx->s_pre));       // the prepare pass's parameter upload has read h_bc
+        u32_rebase(ctx, nblk, nchan, pi.data(), xi.data());
+        u32_chain_end(ctx, nblk, nchan, chain);
+        export_chain(chain, nchan, prn_out, phase_out);
+        if (handoff) handoff(user, prn_out, phase_out);
+        trace(ctx, "handed over");
+        CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, (size_t) nblk * nchan * sizeof(BlockChanDev), cudaMemcpyHostToDevice, sk));
+        st.h2d_bytes += (int64_t) ((size_t) nblk * nchan * sizeof(BlockChanDev));
+        int iseg = 0, ichunk = 0;
+        for (size_t i = 0; i < segs.size(); i++) {
+            const int b0 = segs[i].first, b1 = segs[i].second;
+            SynthArgs a{};
+            fill_args(ctx, a, b0, b1 - b0, nchan, sample_size, (char *) ctx->pending.dst + (size_t) b0 * blk_bytes);
+            ctx->cur_seg = iseg;
+            std::vector<ChainState> seg_end(nchan);
+            int rc = segment_resolve(ctx, b0, b1, nchan, sk, seg_end, st, b0 == 0, a);
+            if (rc) return rc;
+            rc = note_segment_end(ctx, iseg++, b1, nchan, sk, seg_end);
+            if (rc) return rc;
+            CU(cudaEventRecord(ctx->ev_done[ichunk], sk));
+            CU(cudaStreamWaitEvent(s, ctx->ev_done[ichunk], 0));
+            ichunk++;
+            if (ctx->pending.dst_host) {
+                rc = synth_chunks(ctx, b0, b1, nchan, sample_size, ctx->pending.dst, ctx->pending.dst_host, s, st, ichunk);
+                if (rc) return rc;
+            } else {
+                CU(launch_synth(a, s));
+                st.launches += 1;
+            }
+        }
+        ctx->pending.nseg = iseg;
+        CU(cudaEventRecord(ctx->ev[5], s));
+        CU(cudaMemcpyAsync(ctx->h_chain_errors, ctx->d_chain_errors, sizeof(int), cudaMemcpyDeviceToHost, sk));
+        trace(ctx, "checkpoints + synthesis enqueued");
+        return GPSB200_OK;
+    }
     if (ctx->pending.eager) {
         // A successor waits for the outgoing state: scan EVERYTHING first (all probes were submitted up front), hand
         // the exact state on, and only then enqueue the long kernels -- a message sent behind them would wait for them.
@@ -1417,6 +1534,8 @@ int gpsb200_slice_finish_cb(gpsb200_ctx_t *ctx, const int32_t *prn_in, const dou
         return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_finish: call gpsb200_slice_prepare and gpsb200_slice_probe first");
     CU(cudaSetDevice(ctx->cfg.device));
     const int nblk = ctx->pending.nblk, nchan = ctx->pending.nchan;
+    if (!phases_ok(ctx, nchan, prn_in, phase_in))
+        return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_finish: phase_in is not a carrier phase of this context");
     ctx->pending.active = false;
     std::vector<ChainState> chain(nchan);
     seed_chain(chain, nchan, prn_in, phase_in);
@@ -1518,17 +1637,78 @@ int gpsb200_link_apply(const gpsb200_slice_link_t *link, int nchan, const int32_
     return GPSB200_OK;
 }
 
+int gpsb200_slice_link_host_nco(const gpsb200_chan_t *chans, int nblk, int nchan, int carrier_nco,
+                                gpsb200_slice_link_t *link) {
+    if (carrier_nco == GPSB200_CARRIER_FP64) return gpsb200_slice_link_host(chans, nblk, nchan, link);
+    if (carrier_nco != GPSB200_CARRIER_U32 || !chans || !link || nblk < 1 || nchan < 1 || nchan > GPSB200_MAX_CHAN)
+        return GPSB200_ERR_ARG;
+    // exact: the advance of a block is 300000 * carr_phasestep modulo 2^32 (gps.c:2828)
+    memset(link, 0, sizeof *link);
+    for (int c = 0; c < nchan; c++) {
+        uint32_t acc = 0u;
+        int prev = chans[c].prn;
+        bool absolute = false;
+        link->prn_first[c] = prev;
+        link->first_phase[c] = prev > 0 ? chans[c].carr_phase : 0.0;
+        for (int b = 0; b < nblk; b++) {
+            const gpsb200_chan_t &in = chans[(size_t) b * nchan + c];
+            if (in.prn <= 0) {
+                prev = 0;
+                absolute = true;
+                continue;
+            }
+            if (in.prn != prev) {
+                if (!valid_u32_phase(in.carr_phase)) return GPSB200_ERR_ARG;
+                acc = (uint32_t) in.carr_phase;
+                absolute = true;
+            }
+            prev = in.prn;
+            acc += (uint32_t) GPSB200_BLOCK_SAMPLES * (uint32_t) lanes::u32_carrier_step(in.f_carr);
+        }
+        link->prn_last[c] = prev > 0 ? prev : 0;
+        link->reset_inside[c] = absolute ? 1 : 0;
+        link->value[c] = (double) acc;
+    }
+    return GPSB200_OK;
+}
+
+int gpsb200_link_apply_nco(const gpsb200_slice_link_t *link, int nchan, int carrier_nco, const int32_t *prn_in,
+                           const double *phase_in, int32_t *prn_out, double *phase_out) {
+    if (carrier_nco == GPSB200_CARRIER_FP64) return gpsb200_link_apply(link, nchan, prn_in, phase_in, prn_out, phase_out);
+    if (carrier_nco != GPSB200_CARRIER_U32 || !link || !prn_out || !phase_out || nchan < 1 || nchan > GPSB200_MAX_CHAN)
+        return GPSB200_ERR_ARG;
+    for (int c = 0; c < nchan; c++) {
+        if (link->prn_last[c] <= 0) {
+            prn_out[c] = 0;
+            phase_out[c] = 0.0;
+            continue;
+        }
+        uint32_t u = (uint32_t) link->value[c];
+        if (!link->reset_inside[c]) {
+            const bool cont = prn_in && phase_in && prn_in[c] > 0 && prn_in[c] == link->prn_first[c];
+            const double base = cont ? phase_in[c] : link->first_phase[c];
+            if (!valid_u32_phase(base)) return GPSB200_ERR_ARG;
+            u += (uint32_t) base;
+        }
+        prn_out[c] = link->prn_last[c];
+        phase_out[c] = (double) u;
+    }
+    return GPSB200_OK;
+}
+
 const char *gpsb200_synth_kernel_name(const gpsb200_ctx_t *ctx, int nchan) {
     if (!ctx) return "";
     SynthArgs a{};
     a.nchan = nchan;
     a.run_samples = ctx->cfg.run_samples;
     a.lanes = ctx->lanes_on && !ctx->lanes_veto ? 1 : 0;
+    if (ctx->u32) return synth_lanes_applicable(a) ? "k_synth_lanes_u32" : "k_synth_u32";
     return synth_lanes_applicable(a) ? "k_synth_lanes" : "k_synth";
 }
 
 int gpsb200_debug_corrupt_chain(gpsb200_ctx_t *ctx, int on) {
     if (!ctx) return GPSB200_ERR_ARG;
+    if (ctx->u32) return fail(ctx, GPSB200_ERR_ARG, "gpsb200_debug_corrupt_chain: a U32 carrier context has no carrier chain");
     ctx->fault_inject_chain = on != 0;
     return GPSB200_OK;
 }
@@ -1544,6 +1724,7 @@ int gpsb200_carrier_chain_device(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans
     if (phase_in && nblk > 0)
         for (int c = 0; c < nchan; c++)
             if (chans[c].prn > 0) {
+                if (ctx->u32 && !valid_u32_phase(phase_in[c])) return fail(ctx, GPSB200_ERR_ARG, "phase_in: not a u32 phase");
                 chain[c].prn = chans[c].prn;
                 chain[c].phase = phase_in[c];
             }
@@ -1552,6 +1733,10 @@ int gpsb200_carrier_chain_device(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans
         const gpsb200_chan_t *cw = chans + (size_t) w0 * nchan;
         int rc = prepare_blocks(ctx, cw, 0, nw, nchan, chain);
         if (rc) return rc;
+        if (ctx->u32) {             // exact closed form of the prepared records; no device work
+            u32_chain_end(ctx, nw, nchan, chain);
+            continue;
+        }
         const size_t cnt = (size_t) nw * nchan;
         CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, cnt * sizeof(BlockChanDev), cudaMemcpyHostToDevice, s));
         CU(cudaMemcpyAsync(ctx->d_guess, ctx->h_guess, cnt * sizeof(double), cudaMemcpyHostToDevice, s));
@@ -1574,7 +1759,7 @@ int gpsb200_replay_device(gpsb200_ctx_t *ctx, void *dst_device, void *stream_, i
     SynthArgs a = ctx->last;
     if (dst_device) a.out = dst_device;
     if (kernel_mask & 8) CU(launch_tables(a, s));
-    if (kernel_mask & 4) {
+    if ((kernel_mask & 4) && !ctx->u32) {       // a U32 call has no probes to replay
         CU(launch_probe(a, s));
         CU(launch_chain(a, s));
     }

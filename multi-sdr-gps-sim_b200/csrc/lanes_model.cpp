@@ -30,11 +30,15 @@ extern "C" int gpsb200_lanes_model_block(const gpsb200_chan_t *chans, int nchan,
         GPSB200_BLOCK_SAMPLES % run_samples != 0)
         return GPSB200_ERR_ARG;
     const double delt = 1.0 / (double) GPSB200_SAMPLERATE;
+    const bool u32 = (force & 16) != 0;          // GPSB200_CARRIER_U32: exact phases, as k_synth_lanes<.., U32 = true>
     const int nruns = GPSB200_BLOCK_SAMPLES / run_samples, nwin = run_samples / lanes::kWindow;
     std::vector<std::vector<uint32_t>> chipw(nchan, std::vector<uint32_t>(36, 0));
     std::vector<std::vector<int32_t>> tab(nchan, std::vector<int32_t>(512, 0));
     for (int c = 0; c < nchan; c++) {
         if (chans[c].prn <= 0) continue;
+        if (u32 && !(chans[c].carr_phase >= 0.0 && chans[c].carr_phase < 4294967296.0 &&
+                     chans[c].carr_phase == std::floor(chans[c].carr_phase)))
+            return GPSB200_ERR_ARG;
         if (!lanes::code_step_ok(chans[c].f_code * delt)) return GPSB200_ERR_RANGE;
         uint8_t ca[GPSB200_CA_LEN];
         ca_code(chans[c].prn, ca);
@@ -79,8 +83,14 @@ extern "C" int gpsb200_lanes_model_block(const gpsb200_chan_t *chans, int nchan,
                     lanes::exact_signs(an[c], w, chipf, navf, &S[3 * c]);
                     ++cnt[2];
                 }
-                base[c] = lanes::fast_base(st[c]);
-                step[c] = lanes::fast_step(st[c]);
+                if (u32) {       // window record of the U32 variant: (u_run + 96 w step) << 7, step << 7
+                    const uint32_t su = (uint32_t) lanes::u32_carrier_step(chans[c].f_carr);
+                    base[c] = ((uint32_t) x[c] + (uint32_t) (w * lanes::kWindow) * su) << 7;
+                    step[c] = su << 7;
+                } else {
+                    base[c] = lanes::fast_base(st[c]);
+                    step[c] = lanes::fast_step(st[c]);
+                }
             }
             for (int n = 0; n < lanes::kWindow; n++) {
                 const int q = n / 3, rr = n - 3 * q;
@@ -90,7 +100,7 @@ extern "C" int gpsb200_lanes_model_block(const gpsb200_chan_t *chans, int nchan,
                     if (!st[c].active) continue;
                     const uint32_t p = base[c] + (uint32_t) n * step[c];
                     int k = (int) (p >> 23);
-                    if (lanes::fast_risky(p) || (force & 1)) {
+                    if (!u32 && (lanes::fast_risky(p) || (force & 1))) {
                         const uint64_t m = st[c].P + (uint64_t) n * st[c].D;
                         const uint64_t frac = m & ((1ull << 55) - 1);
                         if ((force & 4) || frac < lanes::kBandCarr || frac > (1ull << 55) - lanes::kBandCarr) ++cnt[3];
@@ -116,7 +126,8 @@ extern "C" int gpsb200_lanes_model_block(const gpsb200_chan_t *chans, int nchan,
         for (int c = 0; c < nchan; c++) {
             if (chans[c].prn <= 0) continue;
             int64_t periods = 0, dummy = 0;
-            nco_advance<NCO_CARRIER>(x[c], chans[c].f_carr * delt, run_samples, dummy);
+            if (u32) x[c] = (double) ((uint32_t) x[c] + (uint32_t) run_samples * (uint32_t) lanes::u32_carrier_step(chans[c].f_carr));
+            else nco_advance<NCO_CARRIER>(x[c], chans[c].f_carr * delt, run_samples, dummy);
             nco_advance<NCO_CODE>(y[c], chans[c].f_code * delt, run_samples, periods);
             nav_advance(iword[c], ibit[c], icode[c], periods);
         }

@@ -799,6 +799,8 @@ int build(gpsb200_scenario *S) {
                             const Range rr = pseudo_range(set[sv], io, grx, ref);
                             const double phase_ini = (2.0 * rr.range - r.range) / kLambda;
                             ch.carr_phase = phase_ini - floor(phase_ini);
+                            // integer carrier build (gps.c:2212-2213): the same fraction as a u32 accumulator
+                            if (cfg.carrier_u32) ch.carr_phase = (double) (unsigned int) (512.0 * 65536.0 * ch.carr_phase);
                             break;
                         }
                     if (i < C) allocated[sv] = i;

@@ -178,22 +178,32 @@ __global__ void __launch_bounds__(128) k_checkpoints(SynthArgs a) {
     int b, c;
     if (idx < per_code) {
         if (!map_block_chan(a, idx, b, c)) return;
-        const BlockChanDev p = a.bc[(size_t) b * a.nchan + c];
+        const size_t i = (size_t) b * a.nchan + c;
+        const BlockChanDev p = a.bc[i];
         RunCkpt *ck = a.ck + (size_t) b * a.nruns * a.nchan + c;
         double y = p.code0;
         int iword = p.nav0 & 0xFF, ibit = (p.nav0 >> 8) & 0xFF, icode = (p.nav0 >> 16) & 0xFF;
+        const uint32_t step = (uint32_t) p.step_u32;
         for (int r = 0; r < a.nruns; r++) {
             RunCkpt *o = ck + (size_t) r * a.nchan;
             o->y = y;
             o->nav = (uint32_t) iword | ((uint32_t) ibit << 8) | ((uint32_t) icode << 16);
             o->pad = 0;
+            // U32 carrier (gps.c:2828): exact closed form, modulo 2^32
+            if (a.u32) o->x = p.prn > 0 ? (double) (p.u0 + (uint32_t) (r * a.run_samples) * step) : 0.0;
             if (p.prn <= 0) continue;
             int64_t periods = 0;
             nco_advance<NCO_CODE>(y, p.c_code, a.run_samples, periods);
             nav_advance(iword, ibit, icode, periods);
         }
+        if (a.u32) {
+            const double x_end = p.prn > 0 ? (double) (p.u0 + (uint32_t) kBlockSamples * step) : 0.0;
+            if (a.carr_end) a.carr_end[i] = x_end;
+            if (a.last_end_host && b == a.nblk - 1) a.last_end_host[c] = x_end;
+        }
         return;
     }
+    if (a.u32) return;          // the grid is rounded up to whole CTAs: U32 launches have no carrier threads
     idx -= per_code;
     if (!map_block_chan(a, idx, b, c)) return;
     const size_t i = (size_t) b * a.nchan + c;
@@ -298,7 +308,9 @@ __device__ __forceinline__ int group_sum(int v) {
     }
 }
 
-template <int GROUP, bool IQ16>
+// U32: the reference's integer carrier build (gps.c:2777, 2828): the carrier is a u32 add per sample and the index
+// (u >> 16) & 511 -- no FP64 carrier, no carrier wrap test; the code NCO, NAV bits and the channel sum are unchanged.
+template <int GROUP, bool IQ16, bool U32>
 __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     SynthSmem<GROUP> &sm = *reinterpret_cast<SynthSmem<GROUP> *>(smem_raw);
@@ -362,15 +374,21 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
     if (__ballot_sync(0xFFFFFFFFu, run_ok) == 0) return;
 
     double x = 0.0, y = 0.0, cc = 0.0, dd = 0.0;
+    uint32_t u = 0u, us = 0u;                                 // U32 carrier: phase, step
     int iword = 0, ibit = 0, icode = 0;
     if (active) {
         const RunCkpt k0 = a.ck[((size_t) b * a.nruns + r) * a.nchan + ch];
-        x = k0.x;
+        if (U32) {
+            u = (uint32_t) k0.x;
+            us = (uint32_t) bc[ch].step_u32;
+        } else {
+            x = k0.x;
+        }
         y = k0.y;
         iword = k0.nav & 0xFF;
         ibit = (k0.nav >> 8) & 0xFF;
         icode = (k0.nav >> 16) & 0xFF;
-        cc = bc[ch].c_carr;
+        if (!U32) cc = bc[ch].c_carr;                         // U32: cc = 0, the FP64 carrier never runs
         dd = bc[ch].c_code;
     }
     // floor(x*512) and floor(y) come out of the low mantissa word of a round-toward-zero
@@ -442,7 +460,8 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
         double KY = K52 - (double) j0;
         // table lookup + channel sum of one sample from a VALID (wrapped) NCO state
         auto emit = [&](double xs, double ys) -> int {
-            const int k = __double2loint(__dadd_rz(xs, K43));  // (int) floor(carr_phase*512), gps.c:2775
+            const int k = U32 ? (int) ((u >> 16) & 511u)       // gps.c:2777
+                              : __double2loint(__dadd_rz(xs, K43));  // (int) floor(carr_phase*512), gps.c:2775
             const int rel = __double2loint(__dadd_rz(ys, KY)); // (int) code_phase - j0, gps.c:2817
             const int kk = k ^ ((w8 >> rel) & 0x100);          // dataBit*codeCA == -1  <=>  k += 256 (mod 512)
             int e;
@@ -456,12 +475,17 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
         };
         // one reference step with its wrap / NAV-bit bookkeeping (gps.c:2789-2826)
         auto step_checked = [&](double &xs, double &ys) {
-            xs = __dadd_rn(xs, cc);
-            ys = __dadd_rn(ys, dd);
-            if (xs >= 1.0) xs = __dadd_rn(xs, -1.0);           // gps.c:2823-2826
-            else if (xs < 0.0) {
-                xs = __dadd_rn(xs, 1.0);
-                if (xs >= 1.0) xs = kBelowOne;                // see nco_exact.h: the phase never reads 1.0
+            if (U32) {
+                u += us;                                       // gps.c:2828
+                ys = __dadd_rn(ys, dd);
+            } else {
+                xs = __dadd_rn(xs, cc);
+                ys = __dadd_rn(ys, dd);
+                if (xs >= 1.0) xs = __dadd_rn(xs, -1.0);       // gps.c:2823-2826
+                else if (xs < 0.0) {
+                    xs = __dadd_rn(xs, 1.0);
+                    if (xs >= 1.0) xs = kBelowOne;            // see nco_exact.h: the phase never reads 1.0
+                }
             }
             if (ys >= 1023.0) {                                // gps.c:2791-2813
                 ys = __dadd_rn(ys, -1023.0);
@@ -488,7 +512,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
 #pragma unroll(GROUP == 32 ? 2 : 1)
         for (int g8 = 0; g8 < len; g8 += 8) {
             const int hx = __double2hiint(x), hy = __double2hiint(y);
-            const bool risky = (hx >= thr_x_hi) | (hx <= thr_x_lo) | (hy >= thr_y);
+            const bool risky = U32 ? hy >= thr_y : (hx >= thr_x_hi) | (hx <= thr_x_lo) | (hy >= thr_y);
             if (!__any_sync(0xFFFFFFFFu, risky)) {
 #pragma unroll
                 for (int h = 0; h < 8; h += 4) {
@@ -496,7 +520,8 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
 #pragma unroll
                     for (int i = 0; i < 4; i++) {
                         sv[i] = emit(x, y);
-                        x = __dadd_rn(x, cc);                  // gps.c:2821, no wrap possible
+                        if (U32) u += us;                      // gps.c:2828
+                        else x = __dadd_rn(x, cc);             // gps.c:2821, no wrap possible
                         y = __dadd_rn(y, dd);                  // gps.c:2789, no wrap possible
                     }
                     park(g8 + h, sv[0], sv[1], sv[2], sv[3]);
@@ -508,12 +533,13 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
 #pragma unroll
                     for (int i = 0; i < 4; i++) {
                         sv[i] = emit(x, y);
-                        const double xn = __dadd_rn(x, cc), yn = __dadd_rn(y, dd);
-                        const bool wrap = ((unsigned) __double2hiint(xn) >= 0x3FF00000u) |
+                        const double xn = U32 ? 0.0 : __dadd_rn(x, cc), yn = __dadd_rn(y, dd);
+                        const bool wrap = (!U32 && (unsigned) __double2hiint(xn) >= 0x3FF00000u) |
                                           ((unsigned) __double2hiint(yn) >= 0x408FF800u);
                         if (__any_sync(0xFFFFFFFFu, wrap)) step_checked(x, y);
                         else {
-                            x = xn;
+                            if (U32) u += us;
+                            else x = xn;
                             y = yn;
                         }
                     }
@@ -536,23 +562,22 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 2) k_synth(SynthArgs a) {
 // ---------------------------------------------------------------------------------
 // Launchers
 // ---------------------------------------------------------------------------------
-template <int GROUP>
-static cudaError_t launch_synth_t(const SynthArgs &a, cudaStream_t s) {
+template <int GROUP, bool IQ16, bool U32>
+static cudaError_t launch_synth_k(const SynthArgs &a, cudaStream_t s) {
     const int rpw = 32 / GROUP;
     const int warps = (a.runs_per_cta + rpw - 1) / rpw;
     const size_t smem = sizeof(SynthSmem<GROUP>);
     const int ctas = a.nblk * a.ctas_per_block;
-    cudaError_t e;
-    if (a.iq16) {
-        e = cudaFuncSetAttribute(k_synth<GROUP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-        if (e != cudaSuccess) return e;
-        k_synth<GROUP, true><<<ctas, warps * 32, smem, s>>>(a);
-    } else {
-        e = cudaFuncSetAttribute(k_synth<GROUP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-        if (e != cudaSuccess) return e;
-        k_synth<GROUP, false><<<ctas, warps * 32, smem, s>>>(a);
-    }
+    cudaError_t e = cudaFuncSetAttribute(k_synth<GROUP, IQ16, U32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+    if (e != cudaSuccess) return e;
+    k_synth<GROUP, IQ16, U32><<<ctas, warps * 32, smem, s>>>(a);
     return cudaGetLastError();
+}
+
+template <int GROUP>
+static cudaError_t launch_synth_t(const SynthArgs &a, cudaStream_t s) {
+    if (a.u32) return a.iq16 ? launch_synth_k<GROUP, true, true>(a, s) : launch_synth_k<GROUP, false, true>(a, s);
+    return a.iq16 ? launch_synth_k<GROUP, true, false>(a, s) : launch_synth_k<GROUP, false, false>(a, s);
 }
 
 cudaError_t launch_synth(const SynthArgs &a, cudaStream_t s) {
@@ -580,7 +605,7 @@ cudaError_t launch_tables(const SynthArgs &a, cudaStream_t s) {
 
 cudaError_t launch_checkpoints(const SynthArgs &a, cudaStream_t s) {
     const int nblk_pad = (a.nblk + 31) & ~31;
-    const long total = 2L * nblk_pad * a.nchan;
+    const long total = (a.u32 ? 1L : 2L) * nblk_pad * a.nchan;      // U32: no carrier walk, code threads only
     const int threads = 128;
     k_checkpoints<<<(unsigned) ((total + threads - 1) / threads), threads, 0, s>>>(a);
     return cudaGetLastError();

@@ -20,13 +20,17 @@ struct BlockChanDev {
     int32_t prn;       // 0 = slot unused
     uint32_t nav0;     // iword | ibit << 8 | icode << 16 at the first sample
     int32_t frame;     // NAV frame index
-    int32_t pad[3];
+    // GPSB200_CARRIER_U32 only (zero otherwise): carr_phasestep = (int) round(512.0 * 65536.0 * f_carr * delt)
+    // (gps.c:2746) and the exact u32 carrier phase at the block's first sample (host prefix sum, prepare_blocks)
+    int32_t step_u32;
+    uint32_t u0;
+    int32_t pad;
 };
 static_assert(sizeof(BlockChanDev) == 64, "BlockChanDev layout");
 
 // Exact NCO state at the first sample of a run (run = run_samples consecutive samples).
 struct RunCkpt {
-    double x;          // carrier phase
+    double x;          // carrier phase (U32 contexts: the u32 accumulator as an integer-valued double)
     double y;          // code phase
     uint32_t nav;      // iword | ibit << 8 | icode << 16
     uint32_t pad;
@@ -77,6 +81,9 @@ struct SynthArgs {
     int lanes;                // nonzero: calls of at most 16 channels may use k_synth_lanes (every code step in its range)
     const double *blk_shift;  // [nblk][nchan] host-resolved spans (mode 1): shift of the block against its probe variant
     const int32_t *blk_pick;  // [nblk][nchan] ... which variant; -1: the block has to be walked exactly
+    int u32;                  // nonzero: GPSB200_CARRIER_U32 context -- the carrier is BlockChanDev::u0 + n * step_u32
+                              // modulo 2^32 (RunCkpt::x holds the run start's u32 phase); every kernel of the call
+                              // picks its carrier variant from this one flag
 };
 
 // Gain-scaled carrier tables of every block (gps.c:2781-2782), fetched by k_synth with TMA bulk copies.
@@ -85,7 +92,8 @@ cudaError_t launch_tables(const SynthArgs &a, cudaStream_t s);
 cudaError_t launch_probe(const SynthArgs &a, cudaStream_t s);
 // Speculative chaining of the block probes inside every span, both parity variants (nco_exact.h: span_chain).
 cudaError_t launch_chain(const SynthArgs &a, cudaStream_t s);
-// Run-start checkpoints for every (block, channel): exact walk, O(#binade crossings).
+// Run-start checkpoints for every (block, channel): exact walk, O(#binade crossings); with a.u32 the code NCO only
+// (one thread per (block, channel)), the carrier value of a run start is the closed form.
 cudaError_t launch_checkpoints(const SynthArgs &a, cudaStream_t s);
 // The per-sample synthesis (gps.c:2767-2857): lanes = channels, warp-sum over channels.
 cudaError_t launch_synth(const SynthArgs &a, cudaStream_t s);

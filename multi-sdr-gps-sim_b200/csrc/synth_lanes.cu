@@ -58,7 +58,12 @@ __device__ __forceinline__ uint64_t shfl64(uint64_t v, int src) {
     return ((uint64_t) hi << 32) | lo;
 }
 
-template <bool IQ16, int CH>
+// U32: the reference's integer carrier build (gps.c:2777, 2828). Sample n of a run has the EXACT phase u_run + n * step
+// (mod 2^32), so the window record carries (u_run + 96 w step) << 7 and the sample side adds n * (step << 7): the index
+// (u >> 16) & 511 lands in bits 23..31 as in the FP64 variant, and the chip sign folds in as bit 31 the same way. What
+// only the FP64 carrier needs is compiled out: the 64-bit linear phase (ChanRun::P/D is then dead), the band tracking
+// (VIMNMX3), the per-window vote and the repair.
+template <bool IQ16, int CH, bool U32>
 __global__ void __launch_bounds__(kLaneWarps * 32, 2) k_synth_lanes(SynthArgs a) {
     constexpr int WINS = 32 / CH;                     // windows per trip
     constexpr int SWZ = 32 / CH;                      // swz(c) = c * SWZ
@@ -132,8 +137,14 @@ __global__ void __launch_bounds__(kLaneWarps * 32, 2) k_synth_lanes(SynthArgs a)
         }
         lanes::init_run(s, chan_ok, an.x0, an.y0, an.navpos, an.c, an.d, navf);
         if (!chan_ok) s.P = s.D = s.Y = s.E = 0;
-        if (half == 0) sm.step[warp][ch] = chan_ok ? lanes::fast_step(s) : 0u;
-        if (WINS == 2 && chan_ok && half == 1) lanes::advance_window(s, navf);
+        // U32 carrier of this lane's channel: phase << 7 at the current window start, step << 7
+        const uint32_t ust = U32 && chan_ok ? (uint32_t) bc[ch].step_u32 << 7 : 0u;
+        uint32_t ub = U32 && chan_ok ? (uint32_t) an.x0 << 7 : 0u;
+        if (half == 0) sm.step[warp][ch] = chan_ok ? (U32 ? ust : lanes::fast_step(s)) : 0u;
+        if (WINS == 2 && chan_ok && half == 1) {
+            lanes::advance_window(s, navf);
+            ub += (uint32_t) lanes::kWindow * ust;
+        }
         const size_t samp0 = (size_t) b * kBlockSamples + (size_t) r * a.run_samples;
 
 #pragma unroll 1
@@ -143,7 +154,7 @@ __global__ void __launch_bounds__(kLaneWarps * 32, 2) k_synth_lanes(SynthArgs a)
                 uint32_t base = 0u;
                 if (chan_ok && w + half < nwin) {
                     if (!lanes::window_signs(s, chipf, navf, S)) lanes::exact_signs(an, w + half, chipf, navf, S);
-                    base = lanes::fast_base(s);
+                    base = U32 ? ub : lanes::fast_base(s);
                 }
                 *reinterpret_cast<uint4 *>(&sm.win[warp][half][ch]) = make_uint4(S[0], S[1], S[2], base);
             }
@@ -185,11 +196,13 @@ __global__ void __launch_bounds__(kLaneWarps * 32, 2) k_synth_lanes(SynthArgs a)
                     acc2 += ea2 + eb2;
                     // fast_risky(p) <=> (~p) << 9 < kBandFast << 9 <=> p << 9 > 0xFFFFFE00 - (kBandFast << 9): the largest
                     // fraction below an index boundary over all channels and samples (the sign bit shifts out)
-                    dmax = __vimax3_u32(dmax, qa0 << 9, qb0 << 9);
-                    dmax = __vimax3_u32(dmax, qa1 << 9, qb1 << 9);
-                    dmax = __vimax3_u32(dmax, qa2 << 9, qb2 << 9);
+                    if (!U32) {
+                        dmax = __vimax3_u32(dmax, qa0 << 9, qb0 << 9);
+                        dmax = __vimax3_u32(dmax, qa1 << 9, qb1 << 9);
+                        dmax = __vimax3_u32(dmax, qa2 << 9, qb2 << 9);
+                    }
                 }
-                if (__any_sync(kFull, dmax > 0xFFFFFE00u - (lanes::kBandFast << 9))) {
+                if (!U32 && __any_sync(kFull, dmax > 0xFFFFFE00u - (lanes::kBandFast << 9))) {
                     // ---- repair: some sample of this window sits within 2^-25 cycles below an index boundary for some
                     // channel. Find the channel(s), take the certain index of exactly those (channel, sample) pairs (64-bit
                     // linear phase; exact walk from the run anchor inside the 2^-41 band) and patch the sums.
@@ -248,6 +261,7 @@ __global__ void __launch_bounds__(kLaneWarps * 32, 2) k_synth_lanes(SynthArgs a)
             if (chan_ok) {
 #pragma unroll
                 for (int i = 0; i < WINS; i++) lanes::advance_window(s, navf);
+                ub += (uint32_t) (WINS * lanes::kWindow) * ust;
             }
         }
     }
@@ -274,20 +288,25 @@ static void lanes_shape(const SynthArgs &a, int *ctas_per_block, int *runs_per_c
     *runs_per_cta = per_cta;
 }
 
-template <bool IQ16, int CH>
+template <bool IQ16, int CH, bool U32>
 static cudaError_t launch_lanes_t(const SynthArgs &a, cudaStream_t s) {
     const size_t smem = lanes_smem_bytes<CH>();
-    cudaError_t e = cudaFuncSetAttribute(k_synth_lanes<IQ16, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+    cudaError_t e = cudaFuncSetAttribute(k_synth_lanes<IQ16, CH, U32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
     if (e != cudaSuccess) return e;
-    k_synth_lanes<IQ16, CH><<<a.nblk * a.ctas_per_block, kLaneWarps * 32, smem, s>>>(a);
+    k_synth_lanes<IQ16, CH, U32><<<a.nblk * a.ctas_per_block, kLaneWarps * 32, smem, s>>>(a);
     return cudaGetLastError();
+}
+
+template <bool U32>
+static cudaError_t launch_lanes_mode(const SynthArgs &a, cudaStream_t s) {
+    if (a.nchan <= 16) return a.iq16 ? launch_lanes_t<true, 16, U32>(a, s) : launch_lanes_t<false, 16, U32>(a, s);
+    return a.iq16 ? launch_lanes_t<true, 32, U32>(a, s) : launch_lanes_t<false, 32, U32>(a, s);
 }
 
 cudaError_t launch_synth_lanes(const SynthArgs &a_in, cudaStream_t s) {
     SynthArgs a = a_in;
     lanes_shape(a, &a.ctas_per_block, &a.runs_per_cta);
-    if (a.nchan <= 16) return a.iq16 ? launch_lanes_t<true, 16>(a, s) : launch_lanes_t<false, 16>(a, s);
-    return a.iq16 ? launch_lanes_t<true, 32>(a, s) : launch_lanes_t<false, 32>(a, s);
+    return a.u32 ? launch_lanes_mode<true>(a, s) : launch_lanes_mode<false>(a, s);
 }
 
 void synth_lanes_launch_shape(const SynthArgs &a, int *ctas, int *threads, size_t *smem) {

@@ -22,6 +22,7 @@
 // point where the accumulated q * delta3 carries. A class word is therefore two shifted copies of the chip stream
 // spliced at that point.
 #pragma once
+#include <math.h>
 #include <stdint.h>
 
 #include "nco_exact.h"
@@ -261,6 +262,11 @@ GPSB_HD int exact_index(uint64_t P, uint64_t D, const Anchor &an, int w, int n, 
 // strictly above it) and the increment per sample, both truncated: sample n's true 32-bit phase lies in
 // (base + n * d1, base + n * d1 + 98), so the index taken from base + n * d1 is right unless its fraction is within
 // kBandFast of the next boundary -- fast_risky().
+// Integer carrier NCO of the reference (GPSB200_CARRIER_U32): carr_phasestep = (int) round(512.0 * 65536.0 * f_carr * delt),
+// gps.c:2746 -- left to right with the constant product folded (two roundings, no FMA), C round (ties away from zero).
+// Host only: the kernels read it from BlockChanDev::step_u32.
+inline int32_t u32_carrier_step(double f_carr) { return (int32_t) round((33554432.0 * f_carr) * (1.0 / 3000000.0)); }
+
 GPSB_HD uint32_t fast_base(const ChanRun &s) { return (uint32_t) (s.P >> 32) - 1u; }
 GPSB_HD uint32_t fast_step(const ChanRun &s) { return (uint32_t) (s.D >> 32); }
 GPSB_HD bool fast_risky(uint32_t p) { return (((~p) << 9) < (kBandFast << 9)); }

@@ -30,7 +30,8 @@
 static void usage() {
     fprintf(stderr,
             "gpsb200-sim -e NAV[.gz] [-3] -l lat,lon,h [-t dist,bearing,height] [-d SEC] [-m motion.csv] [-s y/m/d,h:m:s]\n"
-            "            [--iq16] [-I] [--pluto-gain] [--chan N] [--gpus N] [-o iqdata.bin] [--compat-drop]\n");
+            "            [--iq16] [-I] [--pluto-gain] [--chan N] [--gpus N] [-o iqdata.bin] [--compat-drop] [--u32-carrier]\n"
+            "  --u32-carrier: the stream of the reference built without FLOAT_CARR_PHASE (gps.h:17): integer carrier NCO\n");
     exit(2);
 }
 
@@ -54,7 +55,7 @@ int main(int argc, char **argv) {
     sc.ionosphere_enable = 1;
     sc.max_chan = 12;
     double dur = 300.0;
-    int sample_size = GPSB200_SC08, gpus = 1;
+    int sample_size = GPSB200_SC08, gpus = 1, carrier = GPSB200_CARRIER_FP64;
     bool compat = false;
     std::string out = "iqdata.bin";
     for (int i = 1; i < argc; i++) {
@@ -81,10 +82,12 @@ int main(int argc, char **argv) {
         else if (a == "--gpus") gpus = atoi(need());
         else if (a == "-o") out = need();
         else if (a == "--compat-drop") compat = true;
+        else if (a == "--u32-carrier") carrier = GPSB200_CARRIER_U32;
         else usage();
     }
     if (!sc.nav_file || gpus < 1) usage();
     sc.duration_ds = (int) (dur * 10.0 + 0.5);                  // gps-sim.c:140
+    sc.carrier_u32 = carrier == GPSB200_CARRIER_U32;            // allocation phases of that build (gps.c:2212-2213)
 
     gpsb200_scenario_t *scn = nullptr;
     if (gpsb200_scenario_create(&sc, &scn) != GPSB200_OK) {
@@ -113,6 +116,7 @@ int main(int argc, char **argv) {
         cfg.max_chan = nchan;
         cfg.max_blocks = max_blocks;
         cfg.max_nav_frames = nframes;
+        cfg.carrier_nco = carrier;
         if (gpsb200_create(&cfg, ctx) != GPSB200_OK) {
             fprintf(stderr, "gpsb200: %s\n", gpsb200_last_error(*ctx));
             return false;
@@ -204,7 +208,8 @@ int main(int argc, char **argv) {
             const int base = nblk / gpus, extra = nblk % gpus;
             lo[r + 1] = lo[r] + base + (r < extra ? 1 : 0);
         }
-        // guessed incoming states from the closed-form links: no GPU work, no dependence between the workers
+        // guessed incoming states from the closed-form links (exact with --u32-carrier): no GPU work, no dependence between
+        // the workers
         std::vector<std::vector<int32_t>> gprn(gpus, std::vector<int32_t>(nchan, 0));
         std::vector<std::vector<double>> gph(gpus, std::vector<double>(nchan, 0.0));
         {
@@ -215,8 +220,11 @@ int main(int argc, char **argv) {
                 gprn[r] = p;
                 gph[r] = x;
                 gpsb200_slice_link_t link;
-                if (gpsb200_slice_link_host(chans + (size_t) lo[r] * nchan, lo[r + 1] - lo[r], nchan, &link) != GPSB200_OK) return 1;
-                gpsb200_link_apply(&link, nchan, have ? p.data() : nullptr, have ? x.data() : nullptr, pn.data(), xn.data());
+                if (gpsb200_slice_link_host_nco(chans + (size_t) lo[r] * nchan, lo[r + 1] - lo[r], nchan, carrier, &link) !=
+                    GPSB200_OK)
+                    return 1;
+                gpsb200_link_apply_nco(&link, nchan, carrier, have ? p.data() : nullptr, have ? x.data() : nullptr, pn.data(),
+                                       xn.data());
                 p = pn;
                 x = xn;
                 have = true;
