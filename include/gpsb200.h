@@ -284,7 +284,9 @@ int gpsb200_codegen(int prn, uint8_t ca[GPSB200_CA_LEN]);
  * gps.c:1131-1505, satpos/computeRange/ionosphericDelay gps.c:508-611,1893-2026,
  * computeCodePhase gps.c:2033-2064, eph2sbf/generateNavMsg/computeChecksum gps.c:617-884,
  * 1008-1072,2066-2140, allocateChannel gps.c:2142-2235, the 10 Hz / 30 s loop gps.c:2703-2765,
- * 2870-2932). Almanac pages are not generated (reference run with its almanac disabled). */
+ * 2870-2932). With almanac_file, the almanac pages of subframes 4 and 5 are filled from that SEM file exactly as the
+ * reference fills them from its almanac.sem (almanac_read_file almanac.c:73-184, eph2sbf gps.c:772-884); without it,
+ * the pages are those of the reference run with its almanac disabled. */
 typedef struct gpsb200_scenario_config {
     const char *nav_file;          /* -e: RINEX v2 (or, with rinex3, v3) navigation file */
     const char *motion_file;       /* -m: ECEF motion csv "t,x,y,z" at 10 Hz, NULL = static */
@@ -302,6 +304,12 @@ typedef struct gpsb200_scenario_config {
     int32_t carrier_u32;           /* 1: allocation phases of the reference's integer carrier build (gps.c:2212-2213),
                                       carr_phase = (unsigned int) (512.0 * 65536.0 * frac(phase_ini)); 0: FP64 build */
     double target_distance_m, target_bearing_deg, target_height_m;
+    /* SEM almanac file (the reference's almanac.sem, gps.c:2614-2651), NULL = no almanac pages (the reference with its
+     * almanac disabled). A file that cannot be opened is GPSB200_ERR_ARG; a malformed one is read with the reference's
+     * semantics (a parse error before the end of the file drops the whole almanac). A complete record whose toa is more
+     * than 4 weeks from the start time is GPSB200_ERR_ARG: the reference writes no block then. Added last in version
+     * 0.4: callers must be rebuilt against this header (the struct grew by 8 bytes) */
+    const char *almanac_file;
 } gpsb200_scenario_config_t;
 typedef struct gpsb200_scenario gpsb200_scenario_t;
 

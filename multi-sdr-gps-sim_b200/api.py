@@ -65,7 +65,8 @@ class ScenarioConfig(C.Structure):
                 ("start_year", C.c_int32), ("start_month", C.c_int32), ("start_day", C.c_int32),
                 ("start_hour", C.c_int32), ("start_min", C.c_int32), ("rinex3", C.c_int32),
                 ("start_sec", C.c_double), ("target_valid", C.c_int32), ("carrier_u32", C.c_int32),
-                ("target_distance_m", C.c_double), ("target_bearing_deg", C.c_double), ("target_height_m", C.c_double)]
+                ("target_distance_m", C.c_double), ("target_bearing_deg", C.c_double), ("target_height_m", C.c_double),
+                ("almanac_file", C.c_char_p)]
 
 
 class SliceLink(C.Structure):
@@ -253,10 +254,11 @@ def _u32_step(f_carr):
 
 
 def scenario(nav_file, lat, lon, height, seconds, max_chan=12, motion_file=None, start=None,
-             ionosphere=True, pluto_gain=False, rinex3=False, target=None, carrier="fp64"):
+             ionosphere=True, pluto_gain=False, rinex3=False, target=None, carrier="fp64", almanac=None):
     """Run the host scenario engine. -> (chans[nblk, max_chan] CHAN_DTYPE, nav[nframes, max_chan, 60] uint32).
     start: (y, m, d, hh, mm, sec) or None for the first ephemeris epoch. carrier='u32': allocation phases of the
-    reference's integer carrier build (u32 accumulators)."""
+    reference's integer carrier build (u32 accumulators). almanac: path of a SEM almanac file whose records fill the
+    almanac pages of subframes 4 and 5, as the reference does with its almanac.sem; None: no almanac pages."""
     cfg = ScenarioConfig()
     cfg.nav_file = os.fsencode(nav_file)
     cfg.motion_file = os.fsencode(motion_file) if motion_file else None
@@ -267,6 +269,7 @@ def scenario(nav_file, lat, lon, height, seconds, max_chan=12, motion_file=None,
     cfg.pluto_gain = 1 if pluto_gain else 0
     cfg.rinex3 = 1 if rinex3 else 0
     cfg.carrier_u32 = 1 if carrier_nco(carrier) == CARRIER_U32 else 0
+    cfg.almanac_file = os.fsencode(almanac) if almanac is not None else None
     if target is not None:          # -t distance,bearing,height
         cfg.target_valid = 1
         cfg.target_distance_m, cfg.target_bearing_deg, cfg.target_height_m = [float(v) for v in target]

@@ -1002,7 +1002,7 @@ int run_pipeline(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int nc
 
 extern "C" {
 
-const char *gpsb200_version(void) { return "gpsb200 0.3 (sm_100a)"; }
+const char *gpsb200_version(void) { return "gpsb200 0.4 (sm_100a)"; }
 
 int gpsb200_bind_numa(int device) {
     char bus[32] = {0};

@@ -12,8 +12,10 @@
 // evaluation order (no FMA contraction: -ffp-contract=off) and the same libm calls;
 // tests/test_scenario.py compares every field with the reference's own dumps.
 //
-// Scope notes: almanac pages are not generated (the reference run with its almanac
-// disabled, as in all BASELINE configs); downloads, interactive motion and
+//   SEM almanac reader + almanac pages of subframes 4/5 (almanac.c:73-184, gps.c:772-884),
+//   when a local almanac file is given (the reference's almanac.sem; none = its almanac disabled)
+//
+// Scope notes: almanac downloads (-f), RINEX downloads, interactive motion and
 // the HackRF/Pluto specifics (except the Pluto gain doubling) are out of scope.
 #include <algorithm>
 #include <cmath>
@@ -45,6 +47,10 @@ constexpr double P2_5 = 0.03125, P2_19 = 1.907348632812500e-6, P2_29 = 1.8626451
                  P2_31 = 4.656612873077393e-10, P2_33 = 1.164153218269348e-10, P2_43 = 1.136868377216160e-13,
                  P2_55 = 2.775557561562891e-17, P2_50 = 8.881784197001252e-016, P2_30 = 9.313225746154785e-010,
                  P2_27 = 7.450580596923828e-009, P2_24 = 5.960464477539063e-008;
+// the almanac's scale factors (gps.h:79-84); P2_38 and P2_23 are not exact powers of two, and 2^12 is an int there
+constexpr double P2_21 = 4.76837158203125e-007, P2_38 = 3.63797880709171e-012, P2_11 = 0.00048828125,
+                 P2_23 = 1.19209289550781e-007, P2_20 = 9.5367431640625e-007;
+constexpr int P2p12 = 4096;
 // receiver antenna attenuation in dB per 5 deg of boresight angle (gps.c:215-220)
 const double kAntPatDb[37] = {0.00,  0.00,  0.22,  0.44,  0.67,  1.11,  1.56,  2.00,  2.44,  2.89,  3.56,  4.22,  4.89,
                               5.56,  6.22,  6.89,  7.56,  8.22,  8.89,  9.78,  10.67, 11.56, 12.44, 13.33, 14.44, 15.56,
@@ -84,6 +90,18 @@ struct Channel {
     uint32_t dwrd[GPSB200_NAV_WORDS];
     int ipage = 0, iword = 0, ibit = 0, icode = 0;
     Range rho0;
+};
+// one SEM almanac record (almanac.h:21-37): angles in semicircles, as the file gives them
+struct AlmanacSv {
+    unsigned char ura = 0, health = 0, config_code = 0;
+    unsigned short svid = 0, svn = 0;       // svid != 0: the record was started (its ID line was read)
+    unsigned valid = 0;                     // 1: the record was read to its end
+    double e = 0, delta_i = 0, omegadot = 0, sqrta = 0, omega0 = 0, aop = 0, m0 = 0, af0 = 0, af1 = 0;
+    GpsTime toa;                            // set only when the record is complete
+};
+struct Almanac {
+    unsigned valid = 0;                     // at least one complete record
+    AlmanacSv sv[kMaxSat];
 };
 
 // ---- time (gps.c:315-339, 1094-1124) ---------------------------------------------------
@@ -305,8 +323,81 @@ uint32_t nav_word(uint32_t source, bool nib) {
     return D;
 }
 
-// ---- subframes 1-3 + dummy pages of 4/5 (gps.c:617-884, almanac absent) -----------------------------------
-void build_subframes(const Eph &e, const IonoUtc &io, uint32_t sbf[kSbfPages][kWordsPerSbf]) {
+// ---- SEM almanac reader (almanac.c:73-184) -------------------------------------------------------------------
+// The file is read line by line into a 100-byte buffer (fgets), and every record is written in place as it is
+// parsed, so a partly read record keeps the fields it got. Layout: "n title", "week sec", then min(n - 1, 31) + 1
+// records (unsigned: n = 0 reads 32), each: an optional blank line, ID (0 -> 1, > 32 -> 32; a repeated ID
+// overwrites), SVN (may be blank), URA (capped at 15), "e delta_i omegadot", "sqrta omega0 aop", "m0 af0 af1",
+// health (capped at 63), config (capped at 15). A complete record gets toa = {week + 2048, sec} and valid = 1.
+// A failure before the end of the file drops everything read; a failure at the end of the file keeps it, the
+// record it cut short included (svid set, valid 0). Returns -1 when the file cannot be opened, else 0.
+int read_sem_almanac(const char *path, Almanac &alm) {
+    alm = Almanac();
+    FILE *fp = fopen(path, "rt");
+    if (!fp) return -1;
+    char line[100];
+    auto next = [&]() { return fgets(line, sizeof line, fp) != nullptr; };
+    auto blank = [&]() { return line[0] == '\n' || line[0] == '\r'; };
+    auto parse = [&]() -> bool {
+        unsigned n, week, sec, id;
+        char title[25];
+        if (!next() || sscanf(line, "%u %24s", &n, title) != 2) return false;
+        if (!next() || sscanf(line, "%u %u", &week, &sec) != 2) return false;
+        const unsigned last = std::min(n - 1u, 31u);
+        for (unsigned j = 0; j <= last; j++) {
+            if (!next()) return false;
+            if (blank() && !next()) return false;
+            if (sscanf(line, "%u", &id) != 1) return false;
+            id = std::min(std::max(id, 1u), 32u);
+            AlmanacSv &a = alm.sv[id - 1];
+            a.svid = (unsigned short) id;
+            if (!next()) return false;
+            if (blank()) a.svn = 0;
+            else if (sscanf(line, "%hu", &a.svn) != 1) return false;
+            if (!next() || sscanf(line, "%hhu", &a.ura) != 1) return false;
+            a.ura = std::min<unsigned char>(a.ura, 15);
+            if (!next() || sscanf(line, "%lf %lf %lf", &a.e, &a.delta_i, &a.omegadot) != 3) return false;
+            if (!next() || sscanf(line, "%lf %lf %lf", &a.sqrta, &a.omega0, &a.aop) != 3) return false;
+            if (!next() || sscanf(line, "%lf %lf %lf", &a.m0, &a.af0, &a.af1) != 3) return false;
+            if (!next() || sscanf(line, "%hhu", &a.health) != 1) return false;
+            a.health = std::min<unsigned char>(a.health, 63);
+            if (!next() || sscanf(line, "%hhu", &a.config_code) != 1) return false;
+            a.config_code = std::min<unsigned char>(a.config_code, 15);
+            a.toa.week = (int) week + 2048;     // the file's week is modulo 1024 of the current era
+            a.toa.sec = (double) sec;
+            a.valid = 1;
+            alm.valid = 1;
+        }
+        return true;
+    };
+    if (!parse() && !feof(fp)) alm = Almanac();
+    fclose(fp);
+    return 0;
+}
+
+// one almanac page (subframe 4 pages 2-5 / 7-10, subframe 5 pages 1-24; gps.c:772-863). toa_scaled is toa.sec / 2^12,
+// which the reference spells POW2_12 (an int) in subframe 4 and 4096.0 in subframe 5: the same quotient
+void almanac_page(uint32_t w[kWordsPerSbf], unsigned long subframe, int sv, const AlmanacSv &a, double toa_scaled) {
+    typedef unsigned long UL;
+    const UL dataId = 1, svId = (UL) (sv + 1);
+    const UL ecc = (UL) (a.e / P2_21), toa = (UL) toa_scaled, sqrta = (UL) (a.sqrta / P2_11);
+    const long delta_i = (long) (a.delta_i / P2_19), omegadot = (long) (a.omegadot / P2_38),
+               omega0 = (long) (a.omega0 / P2_23), aop = (long) (a.aop / P2_23), m0 = (long) (a.m0 / P2_23),
+               af0 = (long) (a.af0 / P2_20), af1 = (long) (a.af1 / P2_38);
+    w[0] = (uint32_t) (0x8B0000UL << 6);
+    w[1] = (uint32_t) (subframe << 8);
+    w[2] = (uint32_t) ((dataId << 28) | (svId << 22) | ((ecc & 0xFFFFUL) << 6));
+    w[3] = (uint32_t) (((toa & 0xFFUL) << 22) | ((delta_i & 0xFFFFUL) << 6));
+    w[4] = (uint32_t) ((omegadot & 0xFFFFUL) << 14);            // SV health 0
+    w[5] = (uint32_t) ((sqrta & 0xFFFFFFUL) << 6);
+    w[6] = (uint32_t) ((omega0 & 0xFFFFFFUL) << 6);
+    w[7] = (uint32_t) ((aop & 0xFFFFFFUL) << 6);
+    w[8] = (uint32_t) ((m0 & 0xFFFFFFUL) << 6);
+    w[9] = (uint32_t) (((af0 & 0x7F8UL) << 19) | ((af1 & 0x7FFUL) << 11) | ((af0 & 0x7UL) << 8));
+}
+
+// ---- subframes 1-3 + pages of 4/5 (gps.c:617-884); alm == NULL: the reference with its almanac disabled -----------
+void build_subframes(const Eph &e, const IonoUtc &io, const Almanac *alm, uint32_t sbf[kSbfPages][kWordsPerSbf]) {
     typedef unsigned long UL;    // the reference packs in (64-bit) long; only the low 32 bits survive
     const UL wn = 0, ura = 0, dataId = 1, EMPTY = 0xaaaaaaaaUL;
     const UL toe = (UL) (e.toe.sec / 16.0), toc = (UL) (e.toc.sec / 16.0);
@@ -369,7 +460,18 @@ void build_subframes(const Eph &e, const IonoUtc &io, uint32_t sbf[kSbfPages][kW
             for (int w = 3; w < 9; w++) put(page, w, (EMPTY & 0xFFFFFFUL) << 6);
             put(page, 9, (EMPTY & 0x3FFFFFUL) << 8);
         }
-    if (io.valid) {                                    // subframe 4 page 18: ionosphere + UTC (SV id 56)
+    if (alm) {
+        // subframe 4 pages 2-5 and 7-10: PRN 25-28 and 29-32, for complete records
+        for (int sv = 24; sv < kMaxSat; sv++)
+            if (alm->sv[sv].valid != 0) {
+                const int i = sv <= 27 ? sv - 23 : sv - 22;
+                almanac_page(sbf[3 + i * 2], 0x4UL, sv, alm->sv[sv], alm->sv[sv].toa.sec / P2p12);
+            }
+        // subframe 5 pages 1-24: PRN 1-24, for every record that was started
+        for (int sv = 0; sv < 24; sv++)
+            if (alm->sv[sv].svid != 0) almanac_page(sbf[4 + sv * 2], 0x5UL, sv, alm->sv[sv], alm->sv[sv].toa.sec / 4096.0);
+    }
+    if (io.valid) {                                   // subframe 4 page 18: ionosphere + UTC (SV id 56)
         const int p = 3 + 17 * 2;
         put(p, 0, TLM);
         put(p, 1, 0x4UL << 8);
@@ -391,7 +493,14 @@ void build_subframes(const Eph &e, const IonoUtc &io, uint32_t sbf[kSbfPages][kW
     }
     {                                                   // subframe 5 page 25 (SV id 51): toa / wna
         const int p = 4 + 24 * 2;
-        const UL wna = (UL) (e.toe.week % 256), toa = (UL) (e.toe.sec / 4096.0);
+        // of the first started almanac record (its toa stays {0, 0} when it was cut short), else of the ephemeris
+        UL wna = (UL) (e.toe.week % 256), toa = (UL) (e.toe.sec / 4096.0);
+        for (int sv = 0; alm && sv < kMaxSat; sv++)
+            if (alm->sv[sv].svid != 0) {
+                wna = (UL) (alm->sv[sv].toa.week % 256);
+                toa = (UL) (alm->sv[sv].toa.sec / 4096.0);
+                break;
+            }
         put(p, 0, TLM);
         put(p, 1, 0x5UL << 8);
         put(p, 2, (dataId << 28) | (51UL << 22) | ((toa & 0xFFUL) << 14) | ((wna & 0xFFUL) << 6));
@@ -758,6 +867,24 @@ int build(gpsb200_scenario *S) {
             }
     if (ieph < 0) return fail(S, "no current set of ephemerides");
 
+    // almanac (gps.c:2614-2651): an unreadable file is the caller's error; a malformed one is read as the
+    // reference reads it. A complete record whose toa is more than 4 weeks from the start stops the reference
+    // before its first block.
+    Almanac alm;
+    const bool use_alm = cfg.almanac_file != nullptr;
+    if (use_alm) {
+        if (read_sem_almanac(cfg.almanac_file, alm) != 0) return fail(S, std::string("cannot open almanac file ") + cfg.almanac_file);
+        if (alm.valid)
+            for (int sv = 0; sv < kMaxSat; sv++)
+                if (alm.sv[sv].valid != 0) {
+                    const double dt = gps_diff(alm.sv[sv].toa, g0);
+                    if (dt < -4.0 * kSecWeek || dt > 4.0 * kSecWeek)
+                        return fail(S, "invalid time of almanac: the toa of PRN " + std::to_string(sv + 1) +
+                                           " is more than 4 weeks from the start time");
+                }
+    }
+    const Almanac *almp = use_alm ? &alm : nullptr;
+
     std::vector<Channel> chan(C);
     std::vector<char> fresh(C, 0);                  // slot (re)allocated since the last epoch snapshot
     int allocated[kMaxSat];
@@ -791,7 +918,7 @@ int build(gpsb200_scenario *S) {
                             fresh[i] = 1;
                             // the reference never initialises channel_t.ipage (gps.c:2086 reads it);
                             // its -Og build sees zeroed stack there, which is what is reproduced here
-                            build_subframes(set[sv], io, ch.sbf);
+                            build_subframes(set[sv], io, almp, ch.sbf);
                             build_nav_frame(grx, ch, true);
                             const Range r = pseudo_range(set[sv], io, grx, p0);
                             ch.rho0 = r;
@@ -890,7 +1017,7 @@ int build(gpsb200_scenario *S) {
                         if (gps_diff(eph[ieph + 1][sv].toc, grx) < kSecHour) {
                             ieph++;
                             for (int i = 0; i < C; i++)
-                                if (chan[i].prn != 0) build_subframes(eph[ieph][chan[i].prn - 1], io, chan[i].sbf);
+                                if (chan[i].prn != 0) build_subframes(eph[ieph][chan[i].prn - 1], io, almp, chan[i].sbf);
                         }
                         break;
                     }

@@ -1,5 +1,6 @@
 // gpsb200-sim: file-sink driver with the reference's command-line vocabulary (help.h:20-53:
-// -e nav file, -l location, -t target, -d duration, -m motion file, -s start, --iq16, -I no ionosphere).
+// -e nav file, -l location, -t target, -d duration, -m motion file, -s start, --iq16, -I no ionosphere) and
+// --almanac FILE: the almanac pages the reference builds from its almanac.sem, from a local SEM file.
 // RINEX + location -> scenario engine (host) -> CUDA synthesis -> reference-compatible FIFO ->
 // iqfile writer. Output is byte-identical to the reference's enqueue stream; --compat-drop
 // reproduces the stock program's iqdata.bin (which lacks blocks 1..6, fifo.c:163-168).
@@ -31,6 +32,8 @@ static void usage() {
     fprintf(stderr,
             "gpsb200-sim -e NAV[.gz] [-3] -l lat,lon,h [-t dist,bearing,height] [-d SEC] [-m motion.csv] [-s y/m/d,h:m:s]\n"
             "            [--iq16] [-I] [--pluto-gain] [--chan N] [--gpus N] [-o iqdata.bin] [--compat-drop] [--u32-carrier]\n"
+            "            [--almanac FILE]\n"
+            "  --almanac FILE: SEM almanac for subframes 4/5 (the reference's almanac.sem; without it: no almanac pages)\n"
             "  --u32-carrier: the stream of the reference built without FLOAT_CARR_PHASE (gps.h:17): integer carrier NCO\n");
     exit(2);
 }
@@ -83,6 +86,7 @@ int main(int argc, char **argv) {
         else if (a == "-o") out = need();
         else if (a == "--compat-drop") compat = true;
         else if (a == "--u32-carrier") carrier = GPSB200_CARRIER_U32;
+        else if (a == "--almanac") sc.almanac_file = need();
         else usage();
     }
     if (!sc.nav_file || gpus < 1) usage();
@@ -96,8 +100,9 @@ int main(int argc, char **argv) {
     }
     const int nblk = gpsb200_scenario_blocks(scn), nchan = gpsb200_scenario_channels(scn);
     const int nframes = gpsb200_scenario_nav_frames(scn);
-    fprintf(stderr, "gpsb200-sim: note: no almanac pages are generated -- the stream equals the reference's with its almanac "
-                    "disabled (the reference enables it by default and downloads one)\n");
+    if (!sc.almanac_file)
+        fprintf(stderr, "gpsb200-sim: note: no almanac pages are generated -- the stream equals the reference's with its almanac "
+                        "disabled (the reference enables it by default and downloads one); --almanac FILE adds them\n");
     const gpsb200_chan_t *chans = gpsb200_scenario_chans(scn);
     const uint32_t *nav = gpsb200_scenario_nav(scn);
     const size_t blk_bytes = (size_t) GPSB200_BLOCK_ELEMS * sample_size;
