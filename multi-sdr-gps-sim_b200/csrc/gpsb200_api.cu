@@ -13,6 +13,7 @@
 #include <sched.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -123,7 +124,9 @@ struct gpsb200_ctx {
     gpsb200_config_t cfg{};
     int nruns = 0;
     cudaStream_t s_compute = nullptr, s_copy = nullptr, s_pre = nullptr, s_ck = nullptr;
-    cudaEvent_t ev[8]{};
+    // timing events of a call (gpsb200_stats_t): the call's stream, and the first segment's probe and checkpoint kernels
+    cudaEvent_t ev_start = nullptr, ev_probe_start = nullptr, ev_probe_end = nullptr, ev_ck_start = nullptr,
+                ev_ck_end = nullptr, ev_end = nullptr;
     std::vector<cudaEvent_t> ev_done;      // one per synthesis chunk
     BlockChanDev *d_bc = nullptr, *h_bc = nullptr;
     RunCkpt *d_ck = nullptr, *h_ck = nullptr;          // h_ck: run checkpoints of small calls, computed on the host
@@ -140,26 +143,20 @@ struct gpsb200_ctx {
     CarrierProbe *h_probe = nullptr, *d_probe_host = nullptr;   // ... and in mapped host memory (host fallback)
     CarrierProbe *h_span_sum = nullptr, *d_span_sum = nullptr;  // span summaries, mapped host memory
     SpanBlockState *d_spec = nullptr;                  // speculative block-start phases
-    double *d_run_x = nullptr;                         // run-start states of the block probes' variant trajectories
-    double *d_blk_shift = nullptr, *h_blk_shift = nullptr;     // host-resolved spans: per-block shift / variant pick
-    int32_t *d_blk_pick = nullptr, *h_blk_pick = nullptr;
-    int run_ld = 0;                                    // leading dimension (blocks, padded) of d_run_x
     bool u32 = false;                                  // cfg.carrier_nco == GPSB200_CARRIER_U32: exact closed-form carrier,
                                                        // none of the carrier-chain stages (probes, chaining, scan) run
     bool lanes_on = true;                              // GPSB200_LANES=0: always k_synth (lane = channel)
     bool lanes_veto = false;                           // a channel record outside k_synth_lanes' range was seen
-    int check_stride = 8, check_phase = 0;             // sampled exact re-walk of the chain (GPSB200_CHECK_STRIDE)
     SpanRes *d_span_res = nullptr, *h_span_res = nullptr;
     int max_spans = 0, max_segs = 0;
     double *h_seg_end = nullptr, *d_seg_end = nullptr;   // mapped: device-walked end phases of every pipeline segment's last block
-    int cur_seg = 0;                       // which row of h_seg_end the next checkpoint launch fills
     std::vector<double> seg_expect;        // what the chain says they must be
-    std::vector<cudaEvent_t> ev_seg;       // slice path: probes of segment i complete
+    std::vector<cudaEvent_t> ev_seg;       // probes of segment i complete
     void *const *scatter = nullptr;        // gpsb200_synth_blocks_scatter: one host destination per block
     bool fault_inject_chain = false;
     bool trace_on = false;
     double trace_t0 = 0.0;       // gpsb200_debug_corrupt_chain(): test hook of the device self-check
-    // state of a begun, not yet finished call (gpsb200_synth_begin / _finish)
+    // state of a begun, not yet finished call (gpsb200_slice_prepare / gpsb200_slice_finish)
     struct Pending {
         bool active = false;
         int nblk = 0, nchan = 0, sample_size = 0;
@@ -180,6 +177,10 @@ struct gpsb200_ctx {
 };
 
 namespace {
+
+std::array<cudaEvent_t *, 6> timing_events(gpsb200_ctx *ctx) {
+    return {&ctx->ev_start, &ctx->ev_probe_start, &ctx->ev_probe_end, &ctx->ev_ck_start, &ctx->ev_ck_end, &ctx->ev_end};
+}
 
 struct OneSatellite {          // parameter accessor of span_chain() for the host model: one satellite, increments cc[j]
     const double *cc;
@@ -386,8 +387,10 @@ bool phases_ok(const gpsb200_ctx *ctx, int nchan, const int32_t *prn_in, const d
     return true;
 }
 
-// Second pass of the relative mode: the (guessed) incoming state is known now.
+// Second pass of the relative mode: the (guessed) incoming state is known now. (U32 contexts guess nothing: their
+// start phases are exact and are rebased once the exact incoming state is known, u32_rebase.)
 void finalize_guesses(gpsb200_ctx *ctx, int b0, int b1, int nchan, const int32_t *prn_in, const double *phase_in) {
+    if (ctx->u32) return;
     ctx->pool->run(nchan, [&](int c_lo, int c_hi) {
         for (int c = c_lo; c < c_hi; c++) {
             const BlockChanDev &first = ctx->h_bc[(size_t) b0 * nchan + c];
@@ -430,10 +433,7 @@ void reanchor_guesses(gpsb200_ctx *ctx, int b0, int b1, int nchan, const std::ve
 
 // One block of the chain, resolved on the host from its block probe (the first level of the speculation);
 // the exact sequential walk when the probe cannot be used. Returns 1 when it had to walk.
-inline int resolve_block(ChainState &st, const BlockChanDev &bc, const CarrierProbe &probe, double &start_out,
-                         int32_t &pick_out, double &shift_out) {
-    pick_out = -1;                       // -1: k_checkpoints walks the block exactly
-    shift_out = 0.0;
+inline int resolve_block(ChainState &st, const BlockChanDev &bc, const CarrierProbe &probe, double &start_out) {
     if (bc.prn <= 0) {
         st.prn = 0;
         start_out = 0.0;
@@ -442,12 +442,9 @@ inline int resolve_block(ChainState &st, const BlockChanDev &bc, const CarrierPr
     if (st.prn != bc.prn) st.phase = bc.carr_in;
     st.prn = bc.prn;
     start_out = st.phase;
-    double xe, d;
-    int v;
-    if (carrier_fixup(st.phase, bc.c_carr, probe, xe, &v, &d)) {
+    double xe;
+    if (carrier_fixup(st.phase, bc.c_carr, probe, xe)) {
         st.phase = xe;
-        pick_out = v;
-        shift_out = d;
         return 0;
     }
     int64_t dummy = 0;
@@ -459,10 +456,10 @@ inline int resolve_block(ChainState &st, const BlockChanDev &bc, const CarrierPr
 // carrier_fixup per SPAN from the span summaries k_chain left in mapped host memory; a span the device
 // could not chain speculatively (reallocation inside it, Doppler zero crossing, a rejected block probe)
 // or whose summary does not fit the true start phase is resolved block by block from the block probes.
-// Serial over spans per channel, parallel over channels. Returns the number of blocks walked sequentially.
-int64_t resolve_chain(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<ChainState> &chain,
-                      int64_t *spans_regular, int64_t *spans_slow) {
-    std::vector<int64_t> fallbacks(nchan, 0), reg(nchan, 0), slow(nchan, 0);
+// Serial over spans per channel, parallel over channels. Returns the number of blocks walked sequentially and adds the
+// number of spans resolved block by block to spans_slow.
+int64_t resolve_chain(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<ChainState> &chain, int64_t &spans_slow) {
+    std::vector<int64_t> fallbacks(nchan, 0), slow(nchan, 0);
     const int K = kSpanBlocks;
     const int nspan = (b1 - b0 + K - 1) / K;
     ctx->pool->run(nchan, [&](int c_lo, int c_hi) {
@@ -493,7 +490,6 @@ int64_t resolve_chain(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<C
                         res.variant = v;
                         st.prn = first.prn;
                         st.phase = xe;
-                        ++reg[c];
                         continue;
                     }
                 }
@@ -502,8 +498,7 @@ int64_t resolve_chain(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<C
                 ++slow[c];
                 for (int b = s0; b < s1; b++) {
                     const size_t i = (size_t) b * nchan + c;
-                    fallbacks[c] += resolve_block(st, ctx->h_bc[i], ctx->h_probe[i], ctx->h_carr0[i], ctx->h_blk_pick[i],
-                                                  ctx->h_blk_shift[i]);
+                    fallbacks[c] += resolve_block(st, ctx->h_bc[i], ctx->h_probe[i], ctx->h_carr0[i]);
                 }
             }
             chain[c] = st;
@@ -514,20 +509,23 @@ int64_t resolve_chain(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<C
     if (ctx->fault_inject_chain && b1 - b0 > 6) {
         SpanRes &r = ctx->h_span_res[(size_t) (b0 / K) * nchan];
         if (r.mode == 0) r.shift += 0x1p-51;
-        else if (r.mode == 1) ctx->h_blk_shift[(size_t) (b0 + 5) * nchan] += 0x1p-51;
+        else if (r.mode == 1) ctx->h_carr0[(size_t) (b0 + 5) * nchan] += 0x1p-51;
     }
     int64_t n = 0;
     for (int c = 0; c < nchan; c++) {
         n += fallbacks[c];
-        if (spans_regular) *spans_regular += reg[c];
-        if (spans_slow) *spans_slow += slow[c];
+        spans_slow += slow[c];
     }
     return n;
 }
 
-void fill_args(gpsb200_ctx *ctx, SynthArgs &a, int blk0, int nblk, int nchan, int sample_size, void *out) {
+// Kernel arguments for blocks [blk0, blk1) of a call whose samples go to dst (block 0 of the call; kernels that write no
+// samples need neither dst nor the sample size).
+SynthArgs args_of(gpsb200_ctx *ctx, int blk0, int blk1, int nchan, int sample_size = GPSB200_SC08, void *dst = nullptr) {
     // blk0 is a multiple of kSpanBlocks whenever the chain kernels are launched with these arguments
+    const int nblk = blk1 - blk0;
     const size_t off = (size_t) blk0 * nchan;
+    SynthArgs a{};
     a.bc = ctx->d_bc + off;
     a.carr0 = ctx->d_carr0 + off;
     a.guess = ctx->d_guess + off;
@@ -545,19 +543,12 @@ void fill_args(gpsb200_ctx *ctx, SynthArgs &a, int blk0, int nblk, int nchan, in
     a.atab = ctx->d_atab + (size_t) blk0 * kAtabRows * 32;
     a.carr_end = ctx->d_carr_end + off;
     a.chain_errors = ctx->d_chain_errors;
-    a.out = out;
+    a.out = dst ? (char *) dst + (size_t) blk0 * GPSB200_BLOCK_ELEMS * sample_size : nullptr;
     a.nblk = nblk;
     a.nchan = nchan;
     a.nruns = ctx->nruns;
     a.run_samples = ctx->cfg.run_samples;
     a.iq16 = sample_size == GPSB200_SC16;
-    a.check_stride = ctx->check_stride;
-    a.check_phase = ctx->check_phase;
-    a.run_x = ctx->d_run_x;
-    a.run_b0 = blk0;
-    a.run_ld = ctx->run_ld;
-    a.blk_shift = ctx->d_blk_shift + off;
-    a.blk_pick = ctx->d_blk_pick + off;
     a.lanes = ctx->lanes_on && !ctx->lanes_veto ? 1 : 0;
     a.u32 = ctx->u32 ? 1 : 0;
     // lanes per run follow the channel count; a CTA takes up to 24 warps' worth of runs
@@ -568,6 +559,7 @@ void fill_args(gpsb200_ctx *ctx, SynthArgs &a, int blk0, int nblk, int nchan, in
     per_cta = (ctx->nruns + ctas - 1) / ctas;
     a.runs_per_cta = per_cta;
     a.ctas_per_block = ctas;
+    return a;
 }
 
 int upload_nav(gpsb200_ctx *ctx, cudaStream_t s) {
@@ -584,138 +576,166 @@ int check_call(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int ncha
         (sample_size != GPSB200_SC08 && sample_size != GPSB200_SC16))
         return fail(ctx, GPSB200_ERR_ARG, "bad arguments (1 <= nchan <= cfg.max_chan; 1 <= nblk <= cfg.max_blocks)");
     if (!ctx->s_compute) return fail(ctx, GPSB200_ERR_CUDA, "context has no CUDA device");
-    if (ctx->pending.active) return fail(ctx, GPSB200_ERR_ARG, "a call begun with gpsb200_synth_begin has not been finished");
+    if (ctx->pending.active) return fail(ctx, GPSB200_ERR_ARG, "a call begun with gpsb200_slice_prepare has not been finished");
     CU(cudaSetDevice(ctx->cfg.device));     // the caller may be a thread that never selected the context's device
     return GPSB200_OK;
 }
 
-// Wait for everything this context has in flight (error paths: the caller may free its buffers once it
-// sees the error code, so no copy into them may still be pending).
-void drain(gpsb200_ctx *ctx, cudaStream_t extra) {
+// Wait for everything this context has in flight once a call failed with rc (the caller may free its buffers once it
+// sees the error code, so no copy into them may still be pending); the error text stays that of rc.
+int drained(gpsb200_ctx *ctx, int rc, cudaStream_t extra) {
+    if (rc == GPSB200_OK) return rc;
     if (extra) cudaStreamSynchronize(extra);
     cudaStreamSynchronize(ctx->s_compute);
     cudaStreamSynchronize(ctx->s_pre);
     if (ctx->s_ck) cudaStreamSynchronize(ctx->s_ck);
     cudaStreamSynchronize(ctx->s_copy);
+    return rc;
 }
 
-// First part of a pipeline segment [b0, b1): host records + guesses, parameters up, carrier tables.
-int segment_params(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1, int nchan, int sample_size,
-                   void *dst_dev, cudaStream_t sp, const std::vector<ChainState> &chain, gpsb200_stats_t &st,
-                   SynthArgs &a, gpsb200_slice_link_t *link, std::vector<ChainState> *end_guess = nullptr) {
-    const size_t blk_bytes = (size_t) GPSB200_BLOCK_ELEMS * sample_size;
-    const int nb = b1 - b0;
-    const size_t off = (size_t) b0 * nchan, cnt = (size_t) nb * nchan;
+// The context's own device buffer that results for a host destination are staged in: room for cfg.max_blocks blocks.
+int stage_out(gpsb200_ctx *ctx, int sample_size) {
+    const size_t need = (size_t) ctx->cfg.max_blocks * GPSB200_BLOCK_ELEMS * sample_size;
+    if (ctx->out_bytes >= need) return GPSB200_OK;
+    cudaFree(ctx->d_out);
+    ctx->d_out = nullptr;
+    ctx->out_bytes = 0;
+    CU(cudaMalloc(&ctx->d_out, need));
+    ctx->out_bytes = need;
+    return GPSB200_OK;
+}
+
+// The steps of a pipeline segment [b0, b1), which every driver strings together:
+//   segment_params -> speculate -> scan -> checkpoints -> synthesize.
+
+// Host records + guesses, parameters up, carrier tables.
+int segment_params(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int b0, int b1, int nchan, cudaStream_t sp,
+                   const std::vector<ChainState> &chain, gpsb200_stats_t &st, gpsb200_slice_link_t *link = nullptr,
+                   std::vector<ChainState> *end_guess = nullptr) {
+    const size_t off = (size_t) b0 * nchan, cnt = (size_t) (b1 - b0) * nchan;
     double t0 = now_ms();
     int rc = prepare_blocks(ctx, chans, b0, b1, nchan, chain, link, end_guess);
     if (rc) return rc;
     st.host_chain_ms += now_ms() - t0;
     CU(cudaMemcpyAsync(ctx->d_bc + off, ctx->h_bc + off, cnt * sizeof(BlockChanDev), cudaMemcpyHostToDevice, sp));
-    fill_args(ctx, a, b0, nb, nchan, sample_size, (char *) dst_dev + (size_t) b0 * blk_bytes);
-    CU(launch_tables(a, sp));                        // needs only the parameters: off the chain's critical path
+    CU(launch_tables(args_of(ctx, b0, b1, nchan), sp));     // needs only the parameters: off the chain's critical path
     st.launches += 1;
     st.h2d_bytes += (int64_t) (cnt * sizeof(BlockChanDev));
     return GPSB200_OK;
 }
 
-// Second part: everything speculative -- guesses up, block probes, span chaining. Needs no true start phase.
-int segment_probe(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
-                  const SynthArgs &a) {
-    if (ctx->u32) return GPSB200_OK;                 // exact closed form: nothing to speculate about
+// Everything speculative, on stream sp: guesses up, block probes, span chaining, then `probed` is recorded. Needs no
+// true start phase. A U32 context has nothing to speculate about (exact closed form).
+int speculate(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
+              cudaEvent_t probed) {
+    if (ctx->u32) return GPSB200_OK;
     const size_t off = (size_t) b0 * nchan, cnt = (size_t) (b1 - b0) * nchan;
+    const SynthArgs a = args_of(ctx, b0, b1, nchan);
     CU(cudaMemcpyAsync(ctx->d_guess + off, ctx->h_guess + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
-    if (first) CU(cudaEventRecord(ctx->ev[1], sp));
+    if (first) CU(cudaEventRecord(ctx->ev_probe_start, sp));
     CU(launch_probe(a, sp));
     CU(launch_chain(a, sp));
-    if (first) CU(cudaEventRecord(ctx->ev[2], sp));
+    if (first) CU(cudaEventRecord(ctx->ev_probe_end, sp));
+    CU(cudaEventRecord(probed, sp));
     st.launches += 2;
     st.h2d_bytes += (int64_t) (cnt * sizeof(double));
     st.d2h_bytes += (int64_t) (cnt * sizeof(CarrierProbe) + (size_t) a.nspan * nchan * sizeof(CarrierProbe));
     return GPSB200_OK;
 }
 
-// Second half: wait for the span summaries, host scan from the chain state, resolutions up, exact run
-// checkpoints (+ device self-check). After it the segment's synthesis may be enqueued behind sp.
-int segment_checkpoints(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
-                        const SynthArgs &a, int64_t slow);
-
-int segment_resolve(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, std::vector<ChainState> &chain,
-                    gpsb200_stats_t &st, bool first, const SynthArgs &a, cudaEvent_t probes_done = nullptr,
-                    int64_t *slow_out = nullptr) {
-    if (ctx->u32) {                 // the exact state is a closed form of the prepared records: no probes to wait for
+// Host scan: chain goes from the exact state after block b0-1 to the one after block b1-1, from the probes and span
+// summaries in mapped host memory once `probed` is complete; slow = spans resolved block by block. A U32 context reads
+// the exact state off the prepared records (closed form): there are no probes to wait for.
+int scan(gpsb200_ctx *ctx, int b0, int b1, int nchan, std::vector<ChainState> &chain, gpsb200_stats_t &st,
+         cudaEvent_t probed, int64_t &slow) {
+    slow = 0;
+    if (ctx->u32) {
         u32_chain_end(ctx, b1, nchan, chain);
-        if (slow_out) {
-            *slow_out = 0;
-            return GPSB200_OK;
-        }
-        return segment_checkpoints(ctx, b0, b1, nchan, sp, st, first, a, 0);
-    }
-    // probes and span summaries must be in (mapped) host memory: wait for the segment's own probe event when the
-    // post-scan work runs on a stream of its own (slice path), else for the pre-phase stream
-    if (probes_done) CU(cudaEventSynchronize(probes_done));
-    else CU(cudaStreamSynchronize(sp));
-    const double t0 = now_ms();
-    int64_t reg = 0, slow = 0;
-    st.chain_fallbacks += (int32_t) resolve_chain(ctx, b0, b1, nchan, chain, &reg, &slow);
-    st.host_chain_ms += now_ms() - t0;
-    if (slow_out) {                 // scan only: the caller enqueues the device part later (segment_checkpoints)
-        *slow_out = slow;
         return GPSB200_OK;
     }
-    return segment_checkpoints(ctx, b0, b1, nchan, sp, st, first, a, slow);
+    CU(cudaEventSynchronize(probed));
+    const double t0 = now_ms();
+    st.chain_fallbacks += (int32_t) resolve_chain(ctx, b0, b1, nchan, chain, slow);
+    st.host_chain_ms += now_ms() - t0;
+    return GPSB200_OK;
 }
 
-// Device part of a segment's resolution: resolutions up, exact run checkpoints (+ self-check).
-int segment_checkpoints(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
-                        const SynthArgs &a, int64_t slow) {
+// Device part of the resolution, on stream sp: the scan's resolutions up, exact run checkpoints (+ the per-block
+// self-check). The launch also stores the walked end phases of the segment's last block into row iseg of h_seg_end
+// (mapped memory: a copy-engine transfer would queue behind the large result downloads); chain_after, the scan's state
+// after block b1-1, is what they must be. verify_chain() compares the two: the self-check across segment and call
+// boundaries. After this step the segment's synthesis may be enqueued behind sp.
+int checkpoints(gpsb200_ctx *ctx, int b0, int b1, int nchan, cudaStream_t sp, gpsb200_stats_t &st, bool first,
+                int64_t slow, int iseg, const std::vector<ChainState> &chain_after) {
     const size_t off = (size_t) b0 * nchan, cnt = (size_t) (b1 - b0) * nchan;
+    SynthArgs a = args_of(ctx, b0, b1, nchan);
     const size_t soff = (size_t) (b0 / kSpanBlocks) * nchan, scnt = (size_t) a.nspan * nchan;
-    if (first) CU(cudaEventRecord(ctx->ev[3], sp));
+    if (first) CU(cudaEventRecord(ctx->ev_ck_start, sp));
     if (!ctx->u32) {                                 // U32: k_checkpoints reads no span resolutions
         CU(cudaMemcpyAsync(ctx->d_span_res + soff, ctx->h_span_res + soff, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
         st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
     }
-    if (slow > 0) {                                  // rare: per-block resolutions of the host-resolved spans
+    if (slow > 0) {                                  // rare: per-block start phases of the host-resolved spans
         CU(cudaMemcpyAsync(ctx->d_carr0 + off, ctx->h_carr0 + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
-        CU(cudaMemcpyAsync(ctx->d_blk_shift + off, ctx->h_blk_shift + off, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
-        CU(cudaMemcpyAsync(ctx->d_blk_pick + off, ctx->h_blk_pick + off, cnt * sizeof(int32_t), cudaMemcpyHostToDevice, sp));
-        st.h2d_bytes += (int64_t) (cnt * (2 * sizeof(double) + sizeof(int32_t)));
+        st.h2d_bytes += (int64_t) (cnt * sizeof(double));
     }
-    SynthArgs ack = a;
-    ack.last_end_host = ctx->cur_seg < ctx->max_segs ? ctx->d_seg_end + (size_t) ctx->cur_seg * nchan : nullptr;
-    CU(launch_checkpoints(ack, sp));
-    if (first) CU(cudaEventRecord(ctx->ev[4], sp));
+    const bool noted = iseg < ctx->max_segs;
+    a.last_end_host = noted ? ctx->d_seg_end + (size_t) iseg * nchan : nullptr;
+    CU(launch_checkpoints(a, sp));
+    if (first) CU(cudaEventRecord(ctx->ev_ck_end, sp));
     st.launches += 1;
+    for (int c = 0; noted && c < nchan; c++) {
+        const bool live = chain_after[c].prn > 0 && ctx->h_bc[(size_t) (b1 - 1) * nchan + c].prn == chain_after[c].prn;
+        ctx->seg_expect[(size_t) iseg * nchan + c] = live ? chain_after[c].phase : -1.0;       // -1: nothing to compare
+    }
+    return GPSB200_OK;
+}
+
+// Blocks [b0, b0 + nb) from src (the device copy of block b0) to the host on stream s: into the contiguous buffer
+// dst_host or, when ctx->scatter is set, every block into its own destination.
+int download(gpsb200_ctx *ctx, const char *src, int b0, int nb, int sample_size, void *dst_host, cudaStream_t s,
+             gpsb200_stats_t &st) {
+    const size_t blk_bytes = (size_t) GPSB200_BLOCK_ELEMS * sample_size;
+    if (ctx->scatter) {          // every block straight into its own (FIFO) buffer
+        for (int b = b0; b < b0 + nb; b++)
+            CU(cudaMemcpyAsync(ctx->scatter[b], src + (size_t) (b - b0) * blk_bytes, blk_bytes, cudaMemcpyDeviceToHost, s));
+    } else {
+        CU(cudaMemcpyAsync((char *) dst_host + (size_t) b0 * blk_bytes, src, (size_t) nb * blk_bytes, cudaMemcpyDeviceToHost,
+                           s));
+    }
+    st.d2h_bytes += (int64_t) nb * (int64_t) blk_bytes;
     return GPSB200_OK;
 }
 
 // Synthesis of blocks [b0, b1) in chunks, each chunk's download to dst_host enqueued on s_copy behind it.
-// dst_host is either one contiguous buffer or, when ctx->scatter is set, ignored in favour of one host address per block.
 int synth_chunks(gpsb200_ctx *ctx, int b0, int b1, int nchan, int sample_size, void *dst_dev, void *dst_host,
                  cudaStream_t s, gpsb200_stats_t &st, int &ichunk) {
-    const size_t blk_bytes = (size_t) GPSB200_BLOCK_ELEMS * sample_size;
     // the very first chunks are short, so that the download (the long pole of this path) starts early
     for (int c0 = b0, nc = 0; c0 < b1; c0 += nc, ichunk++) {
         nc = kSynthChunk;
         if (ctx->graded_chunks) nc = c0 == 0 ? 32 : (c0 == 32 ? 96 : (c0 == 128 ? 128 : kSynthChunk));
         nc = std::min(nc, b1 - c0);
-        SynthArgs ac{};
-        char *dout = (char *) dst_dev + (size_t) c0 * blk_bytes;
-        fill_args(ctx, ac, c0, nc, nchan, sample_size, dout);
+        const SynthArgs ac = args_of(ctx, c0, c0 + nc, nchan, sample_size, dst_dev);
         CU(launch_synth(ac, s));
         st.launches += 1;
         CU(cudaEventRecord(ctx->ev_done[ichunk], s));
         CU(cudaStreamWaitEvent(ctx->s_copy, ctx->ev_done[ichunk], 0));
-        if (ctx->scatter) {          // every block straight into its own (FIFO) buffer
-            for (int b = c0; b < c0 + nc; b++)
-                CU(cudaMemcpyAsync(ctx->scatter[b], dout + (size_t) (b - c0) * blk_bytes, blk_bytes, cudaMemcpyDeviceToHost,
-                                   ctx->s_copy));
-        } else {
-            CU(cudaMemcpyAsync((char *) dst_host + (size_t) c0 * blk_bytes, dout, (size_t) nc * blk_bytes,
-                               cudaMemcpyDeviceToHost, ctx->s_copy));
-        }
-        st.d2h_bytes += (int64_t) nc * (int64_t) blk_bytes;
+        const int rc = download(ctx, (const char *) ac.out, c0, nc, sample_size, dst_host, ctx->s_copy, st);
+        if (rc) return rc;
     }
+    return GPSB200_OK;
+}
+
+// Synthesis of the segment on stream s, behind the checkpoints enqueued on sk; with a host destination in chunks whose
+// downloads overlap the synthesis of later chunks.
+int synthesize(gpsb200_ctx *ctx, int b0, int b1, int nchan, int sample_size, void *dst_dev, void *dst_host,
+               cudaStream_t sk, cudaStream_t s, gpsb200_stats_t &st, int &ichunk) {
+    CU(cudaEventRecord(ctx->ev_done[ichunk], sk));
+    CU(cudaStreamWaitEvent(s, ctx->ev_done[ichunk], 0));
+    ichunk++;
+    if (dst_host) return synth_chunks(ctx, b0, b1, nchan, sample_size, dst_dev, dst_host, s, st, ichunk);
+    CU(launch_synth(args_of(ctx, b0, b1, nchan, sample_size, dst_dev), s));
+    st.launches += 1;
     return GPSB200_OK;
 }
 
@@ -775,26 +795,18 @@ int small_call(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int ncha
     rc = upload_nav(ctx, s);
     if (rc) return rc;
     const size_t cnt = (size_t) nblk * nchan;
-    CU(cudaEventRecord(ctx->ev[0], s));
+    CU(cudaEventRecord(ctx->ev_start, s));
     CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, cnt * sizeof(BlockChanDev), cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(ctx->d_ck, ctx->h_ck, cnt * nruns * sizeof(RunCkpt), cudaMemcpyHostToDevice, s));
-    SynthArgs a{};
-    fill_args(ctx, a, 0, nblk, nchan, sample_size, dst_dev);
+    const SynthArgs a = args_of(ctx, 0, nblk, nchan, sample_size, dst_dev);
     CU(launch_tables(a, s));
     CU(launch_synth(a, s));
-    CU(cudaEventRecord(ctx->ev[5], s));
+    CU(cudaEventRecord(ctx->ev_end, s));
     st.launches = 2;
     st.h2d_bytes = (int64_t) (cnt * (sizeof(BlockChanDev) + nruns * sizeof(RunCkpt)));
-    const size_t bytes = (size_t) nblk * GPSB200_BLOCK_ELEMS * sample_size;
     if (dst_host) {
-        if (ctx->scatter) {
-            for (int b = 0; b < nblk; b++)
-                CU(cudaMemcpyAsync(ctx->scatter[b], (char *) dst_dev + (size_t) b * (bytes / nblk), bytes / nblk,
-                                   cudaMemcpyDeviceToHost, s));
-        } else {
-            CU(cudaMemcpyAsync(dst_host, dst_dev, bytes, cudaMemcpyDeviceToHost, s));
-        }
-        st.d2h_bytes = (int64_t) bytes;
+        rc = download(ctx, (const char *) dst_dev, 0, nblk, sample_size, dst_host, s, st);
+        if (rc) return rc;
         CU(cudaStreamSynchronize(s));
     }
     ctx->last = a;
@@ -814,19 +826,6 @@ std::vector<std::pair<int, int>> segments_of(int nblk) {
         b0 = b1;
     }
     return v;
-}
-
-// After the checkpoint kernel of segment i: remember what the chain expects at the segment's end and fetch what the
-// device's exact walk of the segment's last block ended on (k_checkpoints -> carr_end); compared in verify_chain().
-// This extends the device self-check across pipeline-segment (and call) boundaries.
-int note_segment_end(gpsb200_ctx *ctx, int iseg, int b1, int nchan, cudaStream_t sp, const std::vector<ChainState> &chain) {
-    if (iseg >= ctx->max_segs) return GPSB200_OK;
-    for (int c = 0; c < nchan; c++) {
-        const bool live = chain[c].prn > 0 && ctx->h_bc[(size_t) (b1 - 1) * nchan + c].prn == chain[c].prn;
-        ctx->seg_expect[(size_t) iseg * nchan + c] = live ? chain[c].phase : -1.0;       // -1: nothing to compare
-    }
-    (void) sp;       // the checkpoint kernel of the segment stores its last block's end phases into h_seg_end itself
-    return GPSB200_OK;   // (mapped memory: a copy-engine transfer would queue behind the large result downloads)
 }
 
 // Verdict of the device self-check (all of sp's work must be complete): the per-block comparisons inside the
@@ -856,112 +855,70 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
     gpsb200_stats_t st{};
     std::vector<ChainState> chain(nchan);
     seed_chain(chain, nchan, prn_in, phase_in);
-    ctx->check_phase = (ctx->check_phase + 1) % ctx->check_stride;      // the sampled exact re-walk rotates
     ctx->trace_t0 = now_ms();
     trace(ctx, "call");
     if (nblk <= kHostChainBlocks && !ctx->fault_inject_chain)
         return small_call(ctx, chans, nblk, nchan, sample_size, dst_dev, dst_host, s, chain, prn_out, carr_phase_out, stats);
     cudaStream_t sp = ctx->s_pre;                       // stream of the pre-phase
-    CU(cudaEventRecord(ctx->ev[0], s));
-    CU(cudaStreamWaitEvent(sp, ctx->ev[0], 0));         // earlier work on s may still read the buffers rewritten now
+    CU(cudaEventRecord(ctx->ev_start, s));
+    CU(cudaStreamWaitEvent(sp, ctx->ev_start, 0));      // earlier work on s may still read the buffers rewritten now
     int rc = upload_nav(ctx, sp);
     if (rc) return rc;
     CU(cudaMemsetAsync(ctx->d_chain_errors, 0, sizeof(int), sp));
-    int ichunk = 0, iseg = 0;
     const auto segs = segments_of(nblk);
+    const int nseg = (int) segs.size();
+    int ichunk = 0, nverify = nseg;
+    int64_t slow = 0;
     if (!dst_host) {
         // Device destination: nothing has to leave early, so everything speculative goes first -- the host prepares
         // segment after segment (guesses continue from the GUESSED end of the previous segment) while the GPU already
         // probes the earlier ones -- then the host scans the span summaries, and run checkpoints and synthesis are
         // ONE launch each over the whole call.
-        std::vector<ChainState> guess = chain;
-        std::vector<SynthArgs> sa(segs.size());
-        CU(cudaStreamWaitEvent(ctx->s_ck, ctx->ev[0], 0));
-        for (size_t i = 0; i < segs.size(); i++) {
+        std::vector<ChainState> guess = chain, next(nchan);
+        CU(cudaStreamWaitEvent(ctx->s_ck, ctx->ev_start, 0));
+        for (int i = 0; i < nseg; i++) {
             // the segments' walk kernels alternate between two streams: their long tails (walk lengths differ by
             // an order of magnitude between satellites) overlap instead of adding up
             cudaStream_t sw = (i & 1) ? ctx->s_ck : sp;
-            std::vector<ChainState> next(nchan);
-            rc = segment_params(ctx, chans, segs[i].first, segs[i].second, nchan, sample_size, dst_dev, sw, guess, st, sa[i], nullptr,
-                                &next);
+            rc = segment_params(ctx, chans, segs[i].first, segs[i].second, nchan, sw, guess, st, nullptr, &next);
+            if (!rc) rc = speculate(ctx, segs[i].first, segs[i].second, nchan, sw, st, i == 0, ctx->ev_seg[i]);
             if (rc) return rc;
-            rc = segment_probe(ctx, segs[i].first, segs[i].second, nchan, sw, st, i == 0, sa[i]);
-            if (rc) return rc;
-            CU(cudaEventRecord(ctx->ev_seg[std::min((int) i, ctx->max_segs - 1)], sw));
             guess = next;
         }
-        int64_t slow = 0;
         trace(ctx, "speculative work enqueued");
-        if (ctx->u32) chain = guess;                    // U32: the prepared end state is exact
-        for (size_t i = 0; i < segs.size() && !ctx->u32; i++) {
-            CU(cudaEventSynchronize(ctx->ev_seg[std::min((int) i, ctx->max_segs - 1)]));
-            const double t0 = now_ms();
-            int64_t reg = 0, sl = 0;
-            st.chain_fallbacks += (int32_t) resolve_chain(ctx, segs[i].first, segs[i].second, nchan, chain, &reg, &sl);
+        for (int i = 0; i < nseg; i++) {
+            int64_t sl = 0;
+            rc = scan(ctx, segs[i].first, segs[i].second, nchan, chain, st, ctx->ev_seg[i], sl);
+            if (rc) return rc;
             slow += sl;
-            st.host_chain_ms += now_ms() - t0;
         }
         CU(cudaStreamSynchronize(ctx->s_ck));           // (its last segment's event has been waited for; this orders the
         trace(ctx, "host scan done");                   //  checkpoint launch on sp behind everything on s_ck)
-        SynthArgs all{};
-        fill_args(ctx, all, 0, nblk, nchan, sample_size, dst_dev);
-        const size_t cnt = (size_t) nblk * nchan, scnt = (size_t) all.nspan * nchan;
-        CU(cudaEventRecord(ctx->ev[3], sp));
-        if (!ctx->u32) CU(cudaMemcpyAsync(ctx->d_span_res, ctx->h_span_res, scnt * sizeof(SpanRes), cudaMemcpyHostToDevice, sp));
-        if (slow > 0) {
-            CU(cudaMemcpyAsync(ctx->d_carr0, ctx->h_carr0, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
-            CU(cudaMemcpyAsync(ctx->d_blk_shift, ctx->h_blk_shift, cnt * sizeof(double), cudaMemcpyHostToDevice, sp));
-            CU(cudaMemcpyAsync(ctx->d_blk_pick, ctx->h_blk_pick, cnt * sizeof(int32_t), cudaMemcpyHostToDevice, sp));
-        }
-        SynthArgs ack = all;
-        ack.last_end_host = ctx->d_seg_end;
-        CU(launch_checkpoints(ack, sp));
-        CU(cudaEventRecord(ctx->ev[4], sp));
-        rc = note_segment_end(ctx, 0, nblk, nchan, sp, chain);
+        rc = checkpoints(ctx, 0, nblk, nchan, sp, st, true, slow, 0, chain);
+        if (!rc) rc = synthesize(ctx, 0, nblk, nchan, sample_size, dst_dev, nullptr, sp, s, st, ichunk);
         if (rc) return rc;
-        iseg = 1;
-        CU(cudaEventRecord(ctx->ev_done[0], sp));
-        CU(cudaStreamWaitEvent(s, ctx->ev_done[0], 0));
-        CU(launch_synth(all, s));
-        st.launches += 2;
-        if (!ctx->u32) st.h2d_bytes += (int64_t) (scnt * sizeof(SpanRes));
+        nverify = 1;
         trace(ctx, "checkpoints + synthesis enqueued");
-    }
-    for (const auto &sg : segs) {
-        if (!dst_host) break;
-        const int b0 = sg.first, b1 = sg.second;
-        SynthArgs a{};
-        rc = segment_params(ctx, chans, b0, b1, nchan, sample_size, dst_dev, sp, chain, st, a, nullptr);
-        if (rc) return rc;
-        rc = segment_probe(ctx, b0, b1, nchan, sp, st, b0 == 0, a);
-        if (rc) return rc;
-        ctx->cur_seg = iseg;
-        rc = segment_resolve(ctx, b0, b1, nchan, sp, chain, st, b0 == 0, a);
-        if (rc) return rc;
-        rc = note_segment_end(ctx, iseg++, b1, nchan, sp, chain);
-        if (rc) return rc;
-        CU(cudaEventRecord(ctx->ev_done[ichunk], sp));   // synthesis of this segment waits for its checkpoints
-        CU(cudaStreamWaitEvent(s, ctx->ev_done[ichunk], 0));
-        ichunk++;
-        if (!dst_host) {
-            CU(launch_synth(a, s));
-            st.launches += 1;
-        } else {
-            rc = synth_chunks(ctx, b0, b1, nchan, sample_size, dst_dev, dst_host, s, st, ichunk);
+    } else {
+        for (int i = 0; i < nseg; i++) {
+            const int b0 = segs[i].first, b1 = segs[i].second;
+            rc = segment_params(ctx, chans, b0, b1, nchan, sp, chain, st);
+            if (!rc) rc = speculate(ctx, b0, b1, nchan, sp, st, i == 0, ctx->ev_seg[i]);
+            if (!rc) rc = scan(ctx, b0, b1, nchan, chain, st, ctx->ev_seg[i], slow);
+            if (!rc) rc = checkpoints(ctx, b0, b1, nchan, sp, st, i == 0, slow, i, chain);
+            if (!rc) rc = synthesize(ctx, b0, b1, nchan, sample_size, dst_dev, dst_host, sp, s, st, ichunk);
             if (rc) return rc;
         }
     }
-    CU(cudaEventRecord(ctx->ev[5], s));
-    SynthArgs all{};
-    fill_args(ctx, all, 0, nblk, nchan, sample_size, dst_dev);
-    ctx->last = all;
+    CU(cudaEventRecord(ctx->ev_end, s));
+    ctx->last = args_of(ctx, 0, nblk, nchan, sample_size, dst_dev);
     ctx->have_last = true;
     export_chain(chain, nchan, prn_out, carr_phase_out);
     // the device self-check of the carrier chain is never skipped: a wrong start phase must not produce samples silently
     CU(cudaMemcpyAsync(ctx->h_chain_errors, ctx->d_chain_errors, sizeof(int), cudaMemcpyDeviceToHost, sp));
     CU(cudaStreamSynchronize(sp));
     trace(ctx, "pre-phase stream drained (self-check read)");
-    rc = verify_chain(ctx, iseg, nchan);
+    rc = verify_chain(ctx, nverify, nchan);
     if (rc) return rc;
     if (dst_host) {
         CU(cudaStreamSynchronize(s));
@@ -971,13 +928,13 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
         float ms = 0;
         // per-kernel times of the FIRST segment ...
         if (!ctx->u32) {    // (a U32 call records no probe events)
-            cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]);
+            cudaEventElapsedTime(&ms, ctx->ev_probe_start, ctx->ev_probe_end);
             st.probe_kernel_ms = ms;
         }
-        cudaEventElapsedTime(&ms, ctx->ev[3], ctx->ev[4]);
+        cudaEventElapsedTime(&ms, ctx->ev_ck_start, ctx->ev_ck_end);
         st.checkpoint_kernel_ms = ms;
         if (dst_host) {      // ... and the whole span of the call's stream (a device-destination call is still running)
-            cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[5]);
+            cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_end);
             st.kernel_ms = ms;
         }
         *stats = st;
@@ -988,14 +945,11 @@ int run_pipeline_inner(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, 
 int run_pipeline(gpsb200_ctx *ctx, const gpsb200_chan_t *chans, int nblk, int nchan, int sample_size,
                  void *dst_dev, void *dst_host, cudaStream_t s, const int32_t *prn_in, const double *phase_in,
                  int32_t *prn_out, double *carr_phase_out, gpsb200_stats_t *stats) {
-    const int rc = run_pipeline_inner(ctx, chans, nblk, nchan, sample_size, dst_dev, dst_host, s, prn_in, phase_in, prn_out,
-                                      carr_phase_out, stats);
-    if (rc) {                       // nothing of this call may still be in flight when the caller sees the error
-        const std::string keep = ctx->err;
-        drain(ctx, s);
-        ctx->err = keep;
-    }
-    return rc;
+    // nothing of this call may still be in flight when the caller sees an error
+    return drained(ctx,
+                   run_pipeline_inner(ctx, chans, nblk, nchan, sample_size, dst_dev, dst_host, s, prn_in, phase_in,
+                                      prn_out, carr_phase_out, stats),
+                   s);
 }
 
 }  // namespace
@@ -1168,7 +1122,7 @@ int gpsb200_create(const gpsb200_config_t *cfg, gpsb200_ctx_t **out) {
         CU(cudaStreamCreateWithPriority(&ctx->s_pre, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&ctx->s_ck, cudaStreamNonBlocking, hi));
     }
-    for (auto &e : ctx->ev) CU(cudaEventCreate(&e));
+    for (cudaEvent_t *e : timing_events(ctx)) CU(cudaEventCreate(e));
     const int nchunk = (c.max_blocks + kSynthChunk - 1) / kSynthChunk + (c.max_blocks + kSegBlocks - 1) / kSegBlocks + 5;
     ctx->ev_done.resize(nchunk);
     for (auto &e : ctx->ev_done) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -1205,20 +1159,6 @@ int gpsb200_create(const gpsb200_config_t *cfg, gpsb200_ctx_t **out) {
     CU(cudaHostAlloc(&ctx->h_span_sum, nsc * sizeof(CarrierProbe), cudaHostAllocMapped));
     CU(cudaHostGetDevicePointer((void **) &ctx->d_span_sum, ctx->h_span_sum, 0));
     CU(cudaMalloc(&ctx->d_spec, nbc * sizeof(SpanBlockState)));
-    // Run-start carrier states taken from the probes' own trajectories (+ resolved shift) instead of a second exact
-    // walk: implemented and exact (GPU suite green with every block cross-checked), but measured on B200 it does not
-    // pay -- stopping the probe walks at the 125 run starts costs k_probe +0.75 ms per 2999 x 32 blocks, while
-    // k_checkpoints is bound by the latency of its longest walk, which sampling does not shorten. Off unless
-    // GPSB200_DERIVED_ANCHORS=1 (then every 8th warp of blocks, rotating, is still re-walked: GPSB200_CHECK_STRIDE).
-    ctx->run_ld = (c.max_blocks + 31) & ~31;
-    if (const char *ev = getenv("GPSB200_DERIVED_ANCHORS"))
-        if (atoi(ev) != 0)
-            CU(cudaMalloc(&ctx->d_run_x, (size_t) ctx->run_ld * c.max_chan * ctx->nruns * 2 * sizeof(double)));
-    CU(cudaMalloc(&ctx->d_blk_shift, nbc * sizeof(double)));
-    CU(cudaHostAlloc(&ctx->h_blk_shift, nbc * sizeof(double), cudaHostAllocDefault));
-    CU(cudaMalloc(&ctx->d_blk_pick, nbc * sizeof(int32_t)));
-    CU(cudaHostAlloc(&ctx->h_blk_pick, nbc * sizeof(int32_t), cudaHostAllocDefault));
-    if (const char *ev = getenv("GPSB200_CHECK_STRIDE")) ctx->check_stride = std::max(1, atoi(ev));
     if (const char *ev = getenv("GPSB200_TRACE")) ctx->trace_on = atoi(ev) != 0;
     if (const char *ev = getenv("GPSB200_LANES")) ctx->lanes_on = atoi(ev) != 0;
     CU(cudaMalloc(&ctx->d_span_res, nsc * sizeof(SpanRes)));
@@ -1264,19 +1204,14 @@ void gpsb200_destroy(gpsb200_ctx_t *ctx) {
     cudaFree(ctx->d_probe);
     cudaFreeHost(ctx->h_span_sum);
     cudaFree(ctx->d_spec);
-    cudaFree(ctx->d_run_x);
-    cudaFree(ctx->d_blk_shift);
-    cudaFreeHost(ctx->h_blk_shift);
-    cudaFree(ctx->d_blk_pick);
-    cudaFreeHost(ctx->h_blk_pick);
     cudaFree(ctx->d_span_res);
     cudaFreeHost(ctx->h_span_res);
     cudaFree(ctx->d_nav);
     cudaFreeHost(ctx->h_nav);
     cudaFree(ctx->d_chips);
     cudaFree(ctx->d_out);
-    for (auto &e : ctx->ev)
-        if (e) cudaEventDestroy(e);
+    for (cudaEvent_t *e : timing_events(ctx))
+        if (*e) cudaEventDestroy(*e);
     for (auto &e : ctx->ev_done)
         if (e) cudaEventDestroy(e);
     for (auto &e : ctx->ev_seg)
@@ -1314,38 +1249,24 @@ int gpsb200_slice_prepare(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans, int n
     int rc = check_call(ctx, chans, nblk, nchan, sample_size, dst_device ? dst_device : dst_host);
     if (rc) return rc;
     if (!dst_device) {                          // host destination only: stage in the context's own device buffer
-        const size_t need = (size_t) ctx->cfg.max_blocks * GPSB200_BLOCK_ELEMS * sample_size;
-        if (ctx->out_bytes < need) {
-            cudaFree(ctx->d_out);
-            ctx->d_out = nullptr;
-            ctx->out_bytes = 0;
-            CU(cudaMalloc(&ctx->d_out, need));
-            ctx->out_bytes = need;
-        }
+        rc = stage_out(ctx, sample_size);
+        if (rc) return rc;
         dst_device = ctx->d_out;
     }
     if (!link) return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_prepare: link is NULL");
     cudaStream_t s = stream_ ? (cudaStream_t) stream_ : ctx->s_compute;
     cudaStream_t sp = ctx->s_pre;
-    ctx->check_phase = (ctx->check_phase + 1) % ctx->check_stride;      // the sampled exact re-walk rotates
-    CU(cudaEventRecord(ctx->ev[0], s));
-    CU(cudaStreamWaitEvent(sp, ctx->ev[0], 0));         // earlier work on s may still read the buffers rewritten now
-    CU(cudaStreamWaitEvent(ctx->s_ck, ctx->ev[0], 0));
+    CU(cudaEventRecord(ctx->ev_start, s));
+    CU(cudaStreamWaitEvent(sp, ctx->ev_start, 0));      // earlier work on s may still read the buffers rewritten now
+    CU(cudaStreamWaitEvent(ctx->s_ck, ctx->ev_start, 0));
     rc = upload_nav(ctx, sp);
     if (rc) return rc;
     CU(cudaMemsetAsync(ctx->d_chain_errors, 0, sizeof(int), sp));
     std::vector<ChainState> none(nchan);
     gpsb200_stats_t st{};
-    SynthArgs a{};
     memset(link, 0, sizeof *link);
-    rc = segment_params(ctx, chans, 0, nblk, nchan, sample_size, dst_device, sp, none, st, a, link);
-    if (rc) {
-        const std::string keep = ctx->err;
-        drain(ctx, s);
-        ctx->err = keep;
-        return rc;
-    }
-    ctx->last = a;
+    rc = drained(ctx, segment_params(ctx, chans, 0, nblk, nchan, sp, none, st, link), s);
+    if (rc) return rc;
     ctx->have_last = false;
     ctx->pending.active = true;
     ctx->pending.probed = false;
@@ -1369,33 +1290,15 @@ int gpsb200_slice_probe(gpsb200_ctx_t *ctx, const int32_t *prn_in, const double 
     if (!phases_ok(ctx, nchan, prn_in, phase_guess_in))
         return fail(ctx, GPSB200_ERR_ARG, "gpsb200_slice_probe: phase_guess_in is not a carrier phase of this context");
     ctx->pending.eager = eager != 0;
-    if (ctx->u32) {                  // exact closed form: nothing speculative to enqueue
-        ctx->pending.probed = true;
-        return GPSB200_OK;
-    }
     const double t0 = now_ms();
     finalize_guesses(ctx, 0, nblk, nchan, prn_in, phase_guess_in);
     ctx->pending.st.host_chain_ms += now_ms() - t0;
-    int rc = GPSB200_OK, iseg = 0;
-    const auto segs = segments_of(nblk);
-    if (ctx->pending.eager) {
-        // everything speculative at once: ONE probe and ONE chaining launch over the whole slice (no per-segment tails)
-        SynthArgs a{};
-        fill_args(ctx, a, 0, nblk, nchan, ctx->pending.sample_size, nullptr);
-        rc = segment_probe(ctx, 0, nblk, nchan, ctx->s_pre, ctx->pending.st, true, a);
-        for (size_t i = 0; !rc && i < segs.size(); i++)
-            if (cudaEventRecord(ctx->ev_seg[i], ctx->s_pre) != cudaSuccess) rc = fail(ctx, GPSB200_ERR_CUDA, "cudaEventRecord");
-    } else {
-        // only the first segment's; the others follow one by one in gpsb200_slice_finish
-        SynthArgs a{};
-        fill_args(ctx, a, segs[0].first, segs[0].second - segs[0].first, nchan, ctx->pending.sample_size, nullptr);
-        rc = segment_probe(ctx, segs[0].first, segs[0].second, nchan, ctx->s_pre, ctx->pending.st, true, a);
-        if (!rc && cudaEventRecord(ctx->ev_seg[iseg++], ctx->s_pre) != cudaSuccess) rc = fail(ctx, GPSB200_ERR_CUDA, "cudaEventRecord");
-    }
+    // eager: everything speculative at once, ONE probe and ONE chaining launch over the whole slice (no per-segment
+    // tails); lazy: only the first segment's, the others follow one by one in gpsb200_slice_finish
+    const int b1 = ctx->pending.eager ? nblk : segments_of(nblk)[0].second;
+    const int rc = drained(ctx, speculate(ctx, 0, b1, nchan, ctx->s_pre, ctx->pending.st, true, ctx->ev_seg[0]),
+                           ctx->pending.stream);
     if (rc) {
-        const std::string keep = ctx->err;
-        drain(ctx, ctx->pending.stream);
-        ctx->err = keep;
         ctx->pending.active = false;
         return rc;
     }
@@ -1407,66 +1310,32 @@ namespace {
 int slice_finish_inner(gpsb200_ctx *ctx, std::vector<ChainState> &chain, gpsb200_stats_t &st, int32_t *prn_out,
                        double *phase_out, gpsb200_handoff_fn handoff, void *user) {
     const int nblk = ctx->pending.nblk, nchan = ctx->pending.nchan, sample_size = ctx->pending.sample_size;
-    const size_t blk_bytes = (size_t) GPSB200_BLOCK_ELEMS * sample_size;
     cudaStream_t s = ctx->pending.stream, sk = ctx->s_ck;
     const auto segs = segments_of(nblk);
-    std::vector<int64_t> slow(segs.size(), 0);
-    std::vector<std::vector<ChainState>> after(segs.size());
+    const int nseg = (int) segs.size();
+    std::vector<int64_t> slow(nseg, 0);
+    std::vector<std::vector<ChainState>> after(nseg);
+    bool eager = ctx->pending.eager;
     ctx->trace_t0 = now_ms();
     trace(ctx, "slice_finish");
     if (ctx->u32) {
-        // The exact outgoing state is a closed form: hand it over at once, then enqueue per segment the corrected
-        // parameters' run checkpoints and the synthesis.
-        std::vector<ChainState> in = chain;
+        // The exact incoming state is known now: rebase the prepared start phases on it. The outgoing state is then a
+        // closed form, so it is handed over at once (eager order).
         std::vector<int32_t> pi(nchan);
         std::vector<double> xi(nchan);
-        export_chain(in, nchan, pi.data(), xi.data());
+        export_chain(chain, nchan, pi.data(), xi.data());
         CU(cudaStreamSynchronize(ctx->s_pre));       // the prepare pass's parameter upload has read h_bc
         u32_rebase(ctx, nblk, nchan, pi.data(), xi.data());
-        u32_chain_end(ctx, nblk, nchan, chain);
-        export_chain(chain, nchan, prn_out, phase_out);
-        if (handoff) handoff(user, prn_out, phase_out);
-        trace(ctx, "handed over");
         CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, (size_t) nblk * nchan * sizeof(BlockChanDev), cudaMemcpyHostToDevice, sk));
         st.h2d_bytes += (int64_t) ((size_t) nblk * nchan * sizeof(BlockChanDev));
-        int iseg = 0, ichunk = 0;
-        for (size_t i = 0; i < segs.size(); i++) {
-            const int b0 = segs[i].first, b1 = segs[i].second;
-            SynthArgs a{};
-            fill_args(ctx, a, b0, b1 - b0, nchan, sample_size, (char *) ctx->pending.dst + (size_t) b0 * blk_bytes);
-            ctx->cur_seg = iseg;
-            std::vector<ChainState> seg_end(nchan);
-            int rc = segment_resolve(ctx, b0, b1, nchan, sk, seg_end, st, b0 == 0, a);
-            if (rc) return rc;
-            rc = note_segment_end(ctx, iseg++, b1, nchan, sk, seg_end);
-            if (rc) return rc;
-            CU(cudaEventRecord(ctx->ev_done[ichunk], sk));
-            CU(cudaStreamWaitEvent(s, ctx->ev_done[ichunk], 0));
-            ichunk++;
-            if (ctx->pending.dst_host) {
-                rc = synth_chunks(ctx, b0, b1, nchan, sample_size, ctx->pending.dst, ctx->pending.dst_host, s, st, ichunk);
-                if (rc) return rc;
-            } else {
-                CU(launch_synth(a, s));
-                st.launches += 1;
-            }
-        }
-        ctx->pending.nseg = iseg;
-        CU(cudaEventRecord(ctx->ev[5], s));
-        CU(cudaMemcpyAsync(ctx->h_chain_errors, ctx->d_chain_errors, sizeof(int), cudaMemcpyDeviceToHost, sk));
-        trace(ctx, "checkpoints + synthesis enqueued");
-        return GPSB200_OK;
+        eager = true;
     }
-    if (ctx->pending.eager) {
+    int rc = GPSB200_OK;
+    if (eager) {
         // A successor waits for the outgoing state: scan EVERYTHING first (all probes were submitted up front), hand
         // the exact state on, and only then enqueue the long kernels -- a message sent behind them would wait for them.
-        for (size_t i = 0; i < segs.size(); i++) {
-            SynthArgs a{};
-            if (i == 0) {
-                CU(cudaEventSynchronize(ctx->ev_seg[0]));
-                trace(ctx, "probes complete");
-            }
-            int rc = segment_resolve(ctx, segs[i].first, segs[i].second, nchan, sk, chain, st, i == 0, a, ctx->ev_seg[i], &slow[i]);
+        for (int i = 0; i < nseg; i++) {
+            rc = scan(ctx, segs[i].first, segs[i].second, nchan, chain, st, ctx->ev_seg[0], slow[i]);
             if (rc) return rc;
             after[i] = chain;
         }
@@ -1475,52 +1344,32 @@ int slice_finish_inner(gpsb200_ctx *ctx, std::vector<ChainState> &chain, gpsb200
         if (handoff) handoff(user, prn_out, phase_out);
         trace(ctx, "handed over");
     }
-    int iseg = 0, ichunk = 0;
-    for (size_t i = 0; i < segs.size(); i++) {
+    for (int i = 0, ichunk = 0; i < nseg; i++) {
         const int b0 = segs[i].first, b1 = segs[i].second;
-        SynthArgs a{};
-        fill_args(ctx, a, b0, b1 - b0, nchan, sample_size, (char *) ctx->pending.dst + (size_t) b0 * blk_bytes);
-        ctx->cur_seg = iseg;
-        int rc;
-        if (ctx->pending.eager) {
-            rc = segment_checkpoints(ctx, b0, b1, nchan, sk, st, b0 == 0, a, slow[i]);
-            if (rc) return rc;
-            rc = note_segment_end(ctx, iseg++, b1, nchan, sk, after[i]);
-        } else {
+        if (!eager) {
             // lazy: host scan of this segment as soon as ITS probes are done; checkpoints on a stream of their own
-            rc = segment_resolve(ctx, b0, b1, nchan, sk, chain, st, b0 == 0, a, ctx->ev_seg[iseg]);
+            rc = scan(ctx, b0, b1, nchan, chain, st, ctx->ev_seg[i], slow[i]);
             if (rc) return rc;
-            rc = note_segment_end(ctx, iseg++, b1, nchan, sk, chain);
+            after[i] = chain;
         }
+        rc = checkpoints(ctx, b0, b1, nchan, sk, st, i == 0, slow[i], i, after[i]);
+        if (!rc) rc = synthesize(ctx, b0, b1, nchan, sample_size, ctx->pending.dst, ctx->pending.dst_host, sk, s, st, ichunk);
         if (rc) return rc;
-        CU(cudaEventRecord(ctx->ev_done[ichunk], sk));
-        CU(cudaStreamWaitEvent(s, ctx->ev_done[ichunk], 0));
-        ichunk++;
-        if (ctx->pending.dst_host) {
-            rc = synth_chunks(ctx, b0, b1, nchan, sample_size, ctx->pending.dst, ctx->pending.dst_host, s, st, ichunk);
-            if (rc) return rc;
-        } else {
-            CU(launch_synth(a, s));
-            st.launches += 1;
-        }
-        if (!ctx->pending.eager && b1 < nblk) {
+        if (!eager && b1 < nblk) {
             // lazy: the next segment's speculative work is submitted only now, BEHIND this segment's synthesis, from
             // guesses re-anchored on the exact state just resolved
             const int n1 = std::min(nblk, b1 + kSegBlocks);
             reanchor_guesses(ctx, b1, n1, nchan, chain);
-            SynthArgs an{};
-            fill_args(ctx, an, b1, n1 - b1, nchan, sample_size, nullptr);
-            rc = segment_probe(ctx, b1, n1, nchan, ctx->s_pre, st, false, an);
+            rc = speculate(ctx, b1, n1, nchan, ctx->s_pre, st, false, ctx->ev_seg[i + 1]);
             if (rc) return rc;
-            CU(cudaEventRecord(ctx->ev_seg[iseg], ctx->s_pre));
         }
     }
-    if (!ctx->pending.eager) {
+    if (!eager) {
         export_chain(chain, nchan, prn_out, phase_out);
         if (handoff) handoff(user, prn_out, phase_out);
     }
-    ctx->pending.nseg = iseg;
-    CU(cudaEventRecord(ctx->ev[5], s));
+    ctx->pending.nseg = nseg;
+    CU(cudaEventRecord(ctx->ev_end, s));
     CU(cudaMemcpyAsync(ctx->h_chain_errors, ctx->d_chain_errors, sizeof(int), cudaMemcpyDeviceToHost, sk));
     trace(ctx, "checkpoints + synthesis enqueued");
     return GPSB200_OK;
@@ -1542,16 +1391,10 @@ int gpsb200_slice_finish_cb(gpsb200_ctx_t *ctx, const int32_t *prn_in, const dou
     gpsb200_stats_t st = ctx->pending.st;
     std::vector<int32_t> po(nchan, 0);
     std::vector<double> xo(nchan, 0.0);
-    const int rc = slice_finish_inner(ctx, chain, st, po.data(), xo.data(), handoff, user);
-    if (rc) {
-        const std::string keep = ctx->err;
-        drain(ctx, ctx->pending.stream);
-        ctx->err = keep;
-        return rc;
-    }
-    SynthArgs all{};
-    fill_args(ctx, all, 0, nblk, nchan, ctx->pending.sample_size, ctx->pending.dst);
-    ctx->last = all;
+    const int rc =
+        drained(ctx, slice_finish_inner(ctx, chain, st, po.data(), xo.data(), handoff, user), ctx->pending.stream);
+    if (rc) return rc;
+    ctx->last = args_of(ctx, 0, nblk, nchan, ctx->pending.sample_size, ctx->pending.dst);
     ctx->have_last = true;
     ctx->pending.finished = true;
     for (int c = 0; c < nchan; c++) {
@@ -1717,10 +1560,11 @@ int gpsb200_carrier_chain_device(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans
                                  const double *phase_in, double *phase_out) {
     if (!ctx || !chans || !phase_out || nblk < 0 || nchan < 1 || nchan > ctx->cfg.max_chan) return GPSB200_ERR_ARG;
     if (!ctx->s_compute) return fail(ctx, GPSB200_ERR_CUDA, "context has no CUDA device");
-    if (ctx->pending.active) return fail(ctx, GPSB200_ERR_ARG, "a call begun with gpsb200_synth_begin has not been finished");
+    if (ctx->pending.active) return fail(ctx, GPSB200_ERR_ARG, "a call begun with gpsb200_slice_prepare has not been finished");
     CU(cudaSetDevice(ctx->cfg.device));
     cudaStream_t s = ctx->s_compute;
     std::vector<ChainState> chain(nchan);
+    gpsb200_stats_t st{};        // (not reported)
     if (phase_in && nblk > 0)
         for (int c = 0; c < nchan; c++)
             if (chans[c].prn > 0) {
@@ -1733,19 +1577,12 @@ int gpsb200_carrier_chain_device(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans
         const gpsb200_chan_t *cw = chans + (size_t) w0 * nchan;
         int rc = prepare_blocks(ctx, cw, 0, nw, nchan, chain);
         if (rc) return rc;
-        if (ctx->u32) {             // exact closed form of the prepared records; no device work
-            u32_chain_end(ctx, nw, nchan, chain);
-            continue;
-        }
-        const size_t cnt = (size_t) nw * nchan;
-        CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, cnt * sizeof(BlockChanDev), cudaMemcpyHostToDevice, s));
-        CU(cudaMemcpyAsync(ctx->d_guess, ctx->h_guess, cnt * sizeof(double), cudaMemcpyHostToDevice, s));
-        SynthArgs a{};
-        fill_args(ctx, a, 0, nw, nchan, GPSB200_SC08, nullptr);
-        CU(launch_probe(a, s));
-        CU(launch_chain(a, s));
-        CU(cudaStreamSynchronize(s));
-        resolve_chain(ctx, 0, nw, nchan, chain, nullptr, nullptr);
+        if (!ctx->u32)              // the probes read the records (a U32 chain is a closed form of them: no device work)
+            CU(cudaMemcpyAsync(ctx->d_bc, ctx->h_bc, (size_t) nw * nchan * sizeof(BlockChanDev), cudaMemcpyHostToDevice, s));
+        int64_t slow = 0;
+        rc = speculate(ctx, 0, nw, nchan, s, st, false, ctx->ev_seg[0]);
+        if (!rc) rc = scan(ctx, 0, nw, nchan, chain, st, ctx->ev_seg[0], slow);
+        if (rc) return rc;
     }
     ctx->have_last = false;
     for (int c = 0; c < nchan; c++) phase_out[c] = chain[c].prn > 0 ? chain[c].phase : 0.0;
@@ -1783,14 +1620,8 @@ int gpsb200_synth_blocks(gpsb200_ctx_t *ctx, const gpsb200_chan_t *chans, int nb
                          void *dst, double *carr_phase_out, gpsb200_stats_t *stats) {
     int rc = check_call(ctx, chans, nblk, nchan, sample_size, dst);
     if (rc) return rc;
-    const size_t need = (size_t) ctx->cfg.max_blocks * GPSB200_BLOCK_ELEMS * sample_size;
-    if (ctx->out_bytes < need) {
-        cudaFree(ctx->d_out);
-        ctx->d_out = nullptr;
-        ctx->out_bytes = 0;
-        CU(cudaMalloc(&ctx->d_out, need));
-        ctx->out_bytes = need;
-    }
+    rc = stage_out(ctx, sample_size);
+    if (rc) return rc;
     return run_pipeline(ctx, chans, nblk, nchan, sample_size, ctx->d_out, dst, ctx->s_compute, nullptr, nullptr, nullptr,
                         carr_phase_out, stats);
 }

@@ -344,12 +344,7 @@ GPSB_HD int64_t carrier_walk(double &x, double c, int64_t n, bool stop_at_wrap, 
 // One parity variant v of the probe (the device runs the two variants in different threads;
 // each repeats the short walk to the first wrap). Fills n_w/x_w (identical for both v) and
 // the v-th end state and margins.
-// run_samples > 0: the variant trajectory's state at every run start s_r = r * run_samples >= n_w (i.e. at or after
-// the first wrap) is stored to run_x[r * run_stride]; entries of earlier runs are left alone (a trajectory from a
-// guessed start is not parallel to the true one before its first wrap: those run starts are walked exactly from the
-// resolved block start, see k_checkpoints).
-GPSB_HD void carrier_probe_variant(double guess, double c, int64_t n, int v, CarrierProbe &o, int run_samples = 0,
-                                   double *run_x = nullptr, size_t run_stride = 0) {
+GPSB_HD void carrier_probe_variant(double guess, double c, int64_t n, int v, CarrierProbe &o) {
     double x = guess;
     bool wrapped = false, ok = true;
     const int64_t nw = carrier_walk(x, c, n, true, wrapped, ok, nullptr, nullptr);
@@ -368,18 +363,7 @@ GPSB_HD void carrier_probe_variant(double guess, double c, int64_t n, int v, Car
     bool w2, ok2;
     // a parity partner that left [0,1) (x_w at the very edge) is simply unusable
     if (!(xv >= 0.0 && xv < 1.0)) mp = mn = 0.0;
-    else if (run_samples <= 0 || !run_x) carrier_walk(xv, c, n - nw, false, w2, ok2, &mp, &mn);
-    else {
-        const WalkConst wc = walk_const(c);
-        int64_t pos = nw;
-        int64_t r = (nw + run_samples - 1) / run_samples;         // first run that starts at or after the first wrap
-        for (; pos < n; r++) {
-            const int64_t stop = r * (int64_t) run_samples < n ? r * (int64_t) run_samples : n;
-            if (stop > pos) carrier_walk_w(xv, wc, stop - pos, false, w2, ok2, &mp, &mn);
-            pos = stop;
-            if (pos < n) run_x[(size_t) r * run_stride] = xv;
-        }
-    }
+    else carrier_walk(xv, c, n - nw, false, w2, ok2, &mp, &mn);
     o.x_end[v] = xv;
     o.m_pos[v] = mp;
     o.m_neg[v] = mn;
@@ -442,8 +426,6 @@ GPSB_HD bool carrier_fixup(double s, double c, const CarrierProbe &p, double &x_
 // span block by block from the block probes.
 struct SpanBlockState {      // per (block, channel), for the span's variants V = 0, 1:
     double start[2];         // speculative start phase of the block
-    double shift[2];         // the block's speculative trajectory = its block probe's variant pick[V] + shift[V]
-    int32_t pick[2];
 };
 
 // probes / blocks: element j of the span lives at index j * stride; param(j, c, prn) yields block j's carrier
@@ -458,8 +440,6 @@ GPSB_HD void span_chain(const CarrierProbe *probes, ParamFn param, int nblk_span
     sum.x_end[V] = sum.m_pos[V] = sum.m_neg[V] = 0.0;
     const CarrierProbe &p0 = probes[0];
     blocks[0].start[V] = guess;
-    blocks[0].shift[V] = 0.0;
-    blocks[0].pick[V] = V;
     double c0;
     int32_t prn0;
     param(0, c0, prn0);
@@ -485,8 +465,6 @@ GPSB_HD void span_chain(const CarrierProbe *probes, ParamFn param, int nblk_span
         if (b < mn) mn = b;
         if (0.5 * pmp < mp) mp = 0.5 * pmp;
         if (0.5 * pmn < mn) mn = 0.5 * pmn;
-        blocks[i].shift[V] = d;
-        blocks[i].pick[V] = v;
         x = xe;
     }
     sum.n_w = p0.n_w;

@@ -98,9 +98,7 @@ __global__ void __launch_bounds__(128) k_probe(SynthArgs a) {
     const BlockChanDev p = a.bc[i];
     CarrierProbe o;
     if (p.prn > 0) {
-        // run-start states of this variant's trajectory go to run_x[r][v][c][run_b0 + b]
-        double *rx = a.run_x ? a.run_x + ((size_t) v * a.nchan + c) * a.run_ld + a.run_b0 + b : nullptr;
-        carrier_probe_variant(a.guess[i], p.c_carr, kBlockSamples, v, o, a.run_samples, rx, (size_t) 2 * a.nchan * a.run_ld);
+        carrier_probe_variant(a.guess[i], p.c_carr, kBlockSamples, v, o);
     } else {
         o.n_w = -1;
         o.x_w = 0.0;
@@ -209,77 +207,24 @@ __global__ void __launch_bounds__(128) k_checkpoints(SynthArgs a) {
     const size_t i = (size_t) b * a.nchan + c;
     const BlockChanDev p = a.bc[i];
     RunCkpt *ck = a.ck + (size_t) b * a.nruns * a.nchan + c;
-    if (p.prn <= 0) {
-        for (int r = 0; r < a.nruns; r++) ck[(size_t) r * a.nchan].x = 0.0;
-        if (a.carr_end) a.carr_end[i] = 0.0;
-        if (a.last_end_host && b == a.nblk - 1) a.last_end_host[c] = 0.0;
-        return;
-    }
-    // How the block was resolved: which variant of its probe the true trajectory runs parallel to, and the shift.
-    const int sp = b / a.span_blocks;
-    const SpanRes res = a.span_res[(size_t) sp * a.nchan + c];
-    const double start = resolved_start(a, b, c);
-    int pick;
-    double shift;
-    bool by_hand = false;
-    if (res.mode == 0) {
-        const SpanBlockState st = a.spec[i];
-        const bool first = b == sp * a.span_blocks;
-        pick = first ? res.variant : st.pick[res.variant];
-        shift = first ? res.shift : st.shift[res.variant] + res.shift;
-    } else {
-        pick = a.blk_pick[i];
-        shift = a.blk_shift[i];
-        by_hand = true;
-    }
-    const CarrierProbe pr = a.probe[i];
-    const bool derived = pick >= 0 && pr.n_w >= 0 && a.run_x != nullptr;
-    // Sampling is per WARP (= 32 consecutive blocks of one channel, see map_block_chan): a walked lane costs its whole
-    // warp the walk. The last block of a launch is always walked: its end phase is compared with the next launch's
-    // chain state.
-    const bool check = !derived || by_hand || b == a.nblk - 1 || a.check_stride <= 1 ||
-                       (((b >> 5) + a.check_phase) % a.check_stride) == 0;
-    double x_end;
-    if (derived) {
-        // run starts before the probe's first wrap: exact walk from the resolved start (no wrap on the way, a handful
-        // of iterations); from the first wrap on: the probe's trajectory plus the shift (exact, see nco_exact.h)
-        const double *rx = a.run_x + ((size_t) pick * a.nchan + c) * a.run_ld + a.run_b0 + b;
-        const size_t rstride = (size_t) 2 * a.nchan * a.run_ld;
-        double x = start;
-        int64_t pos = 0;
+    double x = 0.0;
+    if (p.prn > 0) {
+        // exact walk of the whole block from its resolved start, storing every run start
+        x = resolved_start(a, b, c);
         for (int r = 0; r < a.nruns; r++) {
-            const int64_t s_r = (int64_t) r * a.run_samples;
-            double v;
-            if (s_r < pr.n_w) {
-                int64_t dummy = 0;
-                nco_advance<NCO_CARRIER>(x, p.c_carr, s_r - pos, dummy);
-                pos = s_r;
-                v = x;
-            } else {
-                v = rx[(size_t) r * rstride] + shift;
-            }
-            ck[(size_t) r * a.nchan].x = v;
-        }
-        x_end = pr.x_end[pick] + shift;
-    }
-    if (check) {
-        // exact walk of the whole block from its resolved start
-        double x = start;
-        int bad = 0;
-        for (int r = 0; r < a.nruns; r++) {
-            if (derived) bad |= f64_bits(ck[(size_t) r * a.nchan].x) != f64_bits(x);
-            else ck[(size_t) r * a.nchan].x = x;
+            ck[(size_t) r * a.nchan].x = x;
             int64_t dummy = 0;
             nco_advance<NCO_CARRIER>(x, p.c_carr, a.run_samples, dummy);
         }
-        if (derived) bad |= f64_bits(x_end) != f64_bits(x);
-        x_end = x;
-        // ... which must also BE the start phase resolved for the next block of the same satellite in this launch
-        if (b + 1 < a.nblk && a.bc[i + a.nchan].prn == p.prn && f64_bits(resolved_start(a, b + 1, c)) != f64_bits(x)) bad = 1;
-        if (bad && a.chain_errors) atomicAdd(a.chain_errors, 1);
+        // ... whose end must BE the start phase resolved for the next block of the same satellite in this launch
+        if (b + 1 < a.nblk && a.bc[i + a.nchan].prn == p.prn && f64_bits(resolved_start(a, b + 1, c)) != f64_bits(x) &&
+            a.chain_errors)
+            atomicAdd(a.chain_errors, 1);
+    } else {
+        for (int r = 0; r < a.nruns; r++) ck[(size_t) r * a.nchan].x = 0.0;
     }
-    if (a.carr_end) a.carr_end[i] = x_end;
-    if (a.last_end_host && b == a.nblk - 1) a.last_end_host[c] = x_end;
+    if (a.carr_end) a.carr_end[i] = x;
+    if (a.last_end_host && b == a.nblk - 1) a.last_end_host[c] = x;
 }
 
 // ---------------------------------------------------------------------------------

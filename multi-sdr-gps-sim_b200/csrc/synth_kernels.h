@@ -70,17 +70,7 @@ struct SynthArgs {
     int *chain_errors;        // self-check counter: blocks whose walked end phase != the next block's start phase
     void *out;                // nblk * 600000 int8 or int16
     int nblk, nchan, nruns, run_samples, runs_per_cta, ctas_per_block, iq16;
-    // Run-start carrier states come from the block probes' trajectories (+ the resolved shift); every check_stride-th
-    // block (offset check_phase, rotating from call to call) and every block the host resolved by hand is ALSO walked
-    // exactly from its resolved start, and every run start and the end phase are compared (device self-check).
-    int check_stride, check_phase;
-    double *run_x;            // [nruns][2][nchan][run_ld] run-start states of the block probes' variant trajectories;
-                              // the block index is innermost (the walk kernels' warps are 32 consecutive blocks of one
-                              // channel: coalesced); indexed with the block number within the CONTEXT: run_b0 + b
-    int run_b0, run_ld;
     int lanes;                // nonzero: calls of at most 16 channels may use k_synth_lanes (every code step in its range)
-    const double *blk_shift;  // [nblk][nchan] host-resolved spans (mode 1): shift of the block against its probe variant
-    const int32_t *blk_pick;  // [nblk][nchan] ... which variant; -1: the block has to be walked exactly
     int u32;                  // nonzero: GPSB200_CARRIER_U32 context -- the carrier is BlockChanDev::u0 + n * step_u32
                               // modulo 2^32 (RunCkpt::x holds the run start's u32 phase); every kernel of the call
                               // picks its carrier variant from this one flag

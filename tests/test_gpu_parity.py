@@ -364,31 +364,37 @@ def test_single_block_call_latency_is_far_below_real_time():
 def test_chain_self_check_catches_corruption():
     # defence in depth: k_checkpoints re-derives every block's end phase by an exact walk and compares it
     # with the start phase the two-level speculation resolved for the next block; a corruption by one unit of
-    # the rounding grid (gpsb200_debug_corrupt_chain) must be reported
-    ch, nav = gps.synthetic_chans(12, 32, seed=77)
-    with gps.Context(32, 12) as ctx:
-        ctx.set_nav_frames(nav)
-        good, _ = ctx.synth_blocks(ch, 1)
-        ctx.debug_corrupt_chain(True)
-        with pytest.raises(gps.GpsB200Error) as e:
-            ctx.synth_blocks(ch, 1)
-        assert e.value.code == -5
-        # the device-destination path reports it as well, with or without a stats request
-        import torch
-        dev = torch.empty(12 * gps.BLOCK_ELEMS, dtype=torch.int8, device="cuda")
-        with pytest.raises(gps.GpsB200Error) as e:
-            ctx.synth_blocks_device(ch, 1, dev.data_ptr())
-        assert e.value.code == -5
-        # ... and so does the three-step slice call, at gpsb200_slice_wait
-        ctx.slice_prepare(ch, 1, dev.data_ptr())
-        ctx.slice_probe()
-        ctx.slice_finish()
-        with pytest.raises(gps.GpsB200Error) as e:
-            ctx.slice_wait()
-        assert e.value.code == -5
-        ctx.debug_corrupt_chain(False)
-        again, _ = ctx.synth_blocks(ch, 1)
-        assert np.array_equal(good, again)
+    # the rounding grid (gpsb200_debug_corrupt_chain) must be reported. The hook corrupts the first span of slot 0:
+    # a regular span, resolved from its span summary, and -- slot 0 changes satellite at block 3 -- a span the host
+    # resolved block by block
+    import torch
+    for realloc in (False, True):
+        ch, nav = gps.synthetic_chans(12, 32, seed=77)
+        if realloc:
+            ch["prn"][3:, 0] = ch["prn"][0, 0] % 32 + 1
+            ch["carr_phase"][3, 0] = 0.25
+        with gps.Context(32, 12) as ctx:
+            ctx.set_nav_frames(nav)
+            good, _ = ctx.synth_blocks(ch, 1)
+            ctx.debug_corrupt_chain(True)
+            with pytest.raises(gps.GpsB200Error) as e:
+                ctx.synth_blocks(ch, 1)
+            assert e.value.code == -5, realloc
+            # the device-destination path reports it as well, with or without a stats request
+            dev = torch.empty(12 * gps.BLOCK_ELEMS, dtype=torch.int8, device="cuda")
+            with pytest.raises(gps.GpsB200Error) as e:
+                ctx.synth_blocks_device(ch, 1, dev.data_ptr())
+            assert e.value.code == -5, realloc
+            # ... and so does the three-step slice call, at gpsb200_slice_wait
+            ctx.slice_prepare(ch, 1, dev.data_ptr())
+            ctx.slice_probe()
+            ctx.slice_finish()
+            with pytest.raises(gps.GpsB200Error) as e:
+                ctx.slice_wait()
+            assert e.value.code == -5, realloc
+            ctx.debug_corrupt_chain(False)
+            again, _ = ctx.synth_blocks(ch, 1)
+            assert np.array_equal(good, again)
 
 
 def test_full_size_3600s_32ch_device_path_properties():
